@@ -26,6 +26,12 @@ and the only collective is the 16-byte all-reduce(min) of [incumbent, dual bound
           runs carry the weak-scaling curve (`value`) and the strong-scaling curve of the named frontier.
 
 ``--impl reference`` times only that CPU path (rank 0).
+
+``--dump-outputs DIR`` writes what the last timed step of `value` returned (see dump_outputs), so that two
+builds can be compared output for output on the same inputs.
+
+bench.py writes nothing into the repository (it may be read-only): no bytecode caches, and a library whose
+sources changed since build() is recompiled into a temporary directory.
 """
 from __future__ import annotations
 
@@ -34,8 +40,10 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
+from pathlib import Path
 
 import numpy as np
 
@@ -120,6 +128,29 @@ class Validator:
             ok += int(st == gs and err <= tol)
         return {'checked': len(self.rows), 'ok': ok, 'max_rel_objective_error': worst, 'tolerance': tol,
                 'against': 'bench_data/*_children.npz (HiGHS dual simplex, made offline), compared after the timed region'}
+
+
+DUMP_NODES = 1 << 19          # per-node values of at most this many nodes (4 MB per array)
+DUMP_SAMPLE = 1 << 20         # (coordinate, node) entries of x and of y (8 MB each)
+
+
+def dump_outputs(out_dir, r, B):
+    """Write the result of one solve_batch_device call as float64 DIR/<name>.npy: obj, lower, status, iters
+    and frac of the first min(B, DUMP_NODES) nodes, and x_sample / y_sample, the primal and dual solutions at
+    DUMP_SAMPLE (coordinate, node) pairs drawn with a fixed seed (the full x and y of 2048 C5 nodes take
+    1.2 GB). At most 36 MB in all."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    k = min(B, DUMP_NODES)
+    out = {name: r[name][:k] for name in ('obj', 'lower', 'status', 'iters', 'frac')}
+    rng = np.random.default_rng(0)
+    for name in ('x', 'y'):
+        rows = r[name].shape[0]
+        idx = rng.integers(0, rows, DUMP_SAMPLE), rng.integers(0, B, DUMP_SAMPLE)
+        out[name + '_sample'] = r[name][tuple(torch.from_numpy(i).to(r[name].device) for i in idx)]
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.double().cpu().numpy())
+    log(f'wrote {len(out)} arrays of the last timed step to {out_dir}')
 
 
 def root_by_oracle(d):
@@ -318,7 +349,11 @@ def main():
     ap.add_argument('--named-steps', type=int, default=1)
     ap.add_argument('--named-warmup', type=int, default=0,
                     help='extra warm-up steps of the named leg (it runs warm: after the W + K steps behind `value`)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned as DIR/<name>.npy '
+                         '(float64, about 17 MB at the default batch; rank 0\'s slice)')
     args = ap.parse_args()
+    sys.dont_write_bytecode = True
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -365,10 +400,10 @@ def main():
     dev = torch.device('cuda', local_rank)
     if world > 1:
         dist.init_process_group('nccl', device_id=dev)
-    if local_rank == 0:
-        _build.build_extension()          # no-op when libblp.so is newer than its sources
-    if world > 1:
-        dist.barrier()
+    if _build.is_stale():
+        # sources changed since build(): this run's library goes to a directory that lives as long as main()
+        lib_dir = tempfile.TemporaryDirectory(prefix='blp_bench_')
+        engine._LIB_PATH = _build.build_extension(out=Path(lib_dir.name) / 'libblp.so')
 
     lp = engine.BatchLP(d.A, d.b, d.c, device=local_rank)
     # blp_allreduce_min over the library's own NCCL communicator when world > 1; all ranks or none
@@ -469,6 +504,8 @@ def main():
     ev1.record(ext)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r, B)
     # per-kernel split: the first 1024 iterations of the first W nodes of the last timed slice once
     # more (full batch width) with CUDA events around every k_primal / k_dual launch
     # (blp_opts.profile: no CUDA graph; not part of `value`)

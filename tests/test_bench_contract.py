@@ -56,6 +56,30 @@ def test_root_fixture_is_the_lp_optimum_of_its_workload(name):
     assert abs(dual - root['objective']) <= 1e-7 * scale
 
 
+def test_dump_outputs_is_seeded_float64_and_bounded(tmp_path):
+    """--dump-outputs writes the same sample of the same result twice, in float64, within 64 MB."""
+    import torch
+    n, m, B, ld = 3000, 1000, 100, 128
+    r = dict(obj=torch.randn(ld, dtype=torch.float64), lower=torch.randn(ld, dtype=torch.float64),
+             status=torch.zeros(ld, dtype=torch.int32), iters=torch.arange(ld, dtype=torch.int32),
+             frac=torch.full((ld,), -1, dtype=torch.int32),
+             x=torch.arange(n * ld, dtype=torch.float64).reshape(n, ld),
+             y=torch.arange(m * ld, dtype=torch.float64).reshape(m, ld))
+    bench.dump_outputs(str(tmp_path / 'a'), r, B)
+    bench.dump_outputs(str(tmp_path / 'b'), r, B)
+    names = sorted(os.listdir(tmp_path / 'a'))
+    assert names == sorted(f'{k}.npy' for k in ('obj', 'lower', 'status', 'iters', 'frac', 'x_sample', 'y_sample'))
+    total = 0
+    for f in names:
+        a, b = np.load(tmp_path / 'a' / f), np.load(tmp_path / 'b' / f)
+        assert a.dtype == np.float64 and np.array_equal(a, b), f
+        total += os.path.getsize(tmp_path / 'a' / f)
+    assert total <= 64 << 20
+    assert np.array_equal(np.load(tmp_path / 'a' / 'obj.npy'), r['obj'][:B].numpy())
+    x = np.load(tmp_path / 'a' / 'x_sample.npy')
+    assert x.size == bench.DUMP_SAMPLE and (x % ld < B).all()     # only columns of real nodes
+
+
 def test_product_arm_never_defines_its_workload_with_the_oracle():
     src = open(os.path.join(ROOT, 'bench.py')).read()
     gpu_arm = src[src.index("    from simple_mip_solver_b200.instances import frontier_nodes\n    n, m, B = d.n"):]

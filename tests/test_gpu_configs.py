@@ -219,10 +219,12 @@ def test_config4_shape_exact_vertex_and_gomory_round(blp_lib):
     """SURVEY 8f #1 at the C4 shape (10 000 x 5 000): a single node's LP goes to the wide dual simplex
     (the whole GPU on one node), so BaseNode gets an exact vertex and basis, GMI cuts are generated from
     tableau rows computed on the device, appended, and the LP is re-solved from the previous basis."""
+    import os
     import time
     from simple_mip_solver_b200 import BaseNode
     d = numpy_random_mip(10000, 5000, density=2e-3, seed=2)
-    gold = float(np.load('bench_data/c4_root.npz')['objective'])
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    gold = float(np.load(os.path.join(root, 'bench_data', 'c4_root.npz'))['objective'])
     model = MILPInstance(A=d.A, b=CyLPArray(d.b), c=CyLPArray(d.c), l=CyLPArray(d.l), u=CyLPArray(d.u),
                          sense=['Min', '>='], integerIndices=d.integer_indices, numVars=d.n)
     node = BaseNode(model.lp, model.integerIndices, idx=0)

@@ -1,6 +1,6 @@
 import os, sys, time
 import numpy as np
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 from simple_mip_solver_b200 import engine
 from simple_mip_solver_b200.instances import grumpy_random_mip
 from oracle.highs_lp import HIGHS_INF, HighsLP
