@@ -23,6 +23,8 @@ pivot count and solution agree bit for bit.
   entering  bound flipping ratio test: candidates in order of (ratio rounded to 2^-36, larger
             |alpha| first, smaller index first); a boxed candidate whose flip leaves the row
             infeasible is flipped, the first one that cannot be flipped enters
+  pivot     alpha_q = Binv a_q first; if it disagrees with alpha_r[q] (PIVOT_MISMATCH), refactorise
+            and price again with nothing applied; otherwise the flips, then the basis change
   stop      0 optimal, 1 primal infeasible (no entering column), 3 pivot limit,
             2 unbounded (a variable ends at an artificial bound)
   finish    x_B, y, d recomputed from Binv, one step of iterative refinement on x_B
@@ -67,6 +69,7 @@ class SimplexResult:
     Binv: np.ndarray
     flips: int = 0
     weights: np.ndarray = None
+    refused: int = 0         # pivots refused by the mismatch check (each followed by a refactorisation)
 
 
 def _weights(Binv):
@@ -106,7 +109,11 @@ def _vecmat_rows(v, M):
 
 def dual_simplex(A, b, c, l, u, row_on=None, col_status=None, row_status=None,
                  max_pivots: int = 2147483647, dse: bool = True, bfrt: bool = True,
-                 start: 'SimplexResult' = None) -> SimplexResult:
+                 start: 'SimplexResult' = None, pivot_mismatch: float = PIVOT_MISMATCH,
+                 refactor_every: int = 0) -> SimplexResult:
+    """``pivot_mismatch`` and ``refactor_every`` (0: max(REFACTOR_EVERY, 2 m)) are the two knobs a library
+    built with -DBLP_TUNING reads from BLP_SX_MISMATCH and BLP_SX_REFACTOR_EVERY: a negative threshold refuses
+    every pivot that does not directly follow a factorisation."""
     A = np.asarray(A, dtype=float)
     m, n = A.shape
     N = n + m
@@ -214,8 +221,9 @@ def dual_simplex(A, b, c, l, u, row_on=None, col_status=None, row_status=None,
     xB, _ = primal()
     w = (start.weights.copy() if start is not None else _weights(Binv)) if dse else np.ones(m)
 
-    pivots = flips_total = 0
+    pivots = flips_total = refused = 0
     since_factor = 0
+    refactor_every = refactor_every if refactor_every > 0 else max(REFACTOR_EVERY, 2 * m)
     status = 0
     while True:
         infeas = np.maximum(lo[head] - xB, xB - hi[head])
@@ -238,7 +246,7 @@ def dual_simplex(A, b, c, l, u, row_on=None, col_status=None, row_status=None,
         if pivots >= min(max_pivots, 50 * N + 1000):     # the cap ends a cycling node (no anti-cycling rule)
             status = 3
             break
-        if since_factor >= max(REFACTOR_EVERY, 2 * m):
+        if since_factor >= refactor_every:
             wb = np.zeros(N, bool)
             wb[head] = True
             factor(wb)
@@ -281,6 +289,15 @@ def dual_simplex(A, b, c, l, u, row_on=None, col_status=None, row_status=None,
         if q < 0:
             status = 1
             break
+        aq = A[:, q] if q < n else -np.eye(m)[:, q - n]
+        alpha_q = _matvec_cols(Binv, aq)
+        if since_factor > 0 and abs(alpha_q[r] - alpha_r[q]) > pivot_mismatch * (1.0 + abs(alpha_r[q])):
+            # the two ways to the pivot element disagree: refactorise and price again. Nothing of this
+            # pivot is applied, the bound flips included: a flipped column would rest on the bound its
+            # reduced cost says is wrong, and nothing after the refactorisation would move it back.
+            since_factor = refactor_every
+            refused += 1
+            continue
         if flips:
             delta = np.zeros(N)
             for j in flips:
@@ -289,11 +306,6 @@ def dual_simplex(A, b, c, l, u, row_on=None, col_status=None, row_status=None,
             col = _matvec_cols(A, delta[:n]) - delta[n:]
             xB = xB - _matvec_cols(Binv, col)
             flips_total += len(flips)
-        aq = A[:, q] if q < n else -np.eye(m)[:, q - n]
-        alpha_q = _matvec_cols(Binv, aq)
-        if since_factor > 0 and abs(alpha_q[r] - alpha_r[q]) > PIVOT_MISMATCH * (1.0 + abs(alpha_r[q])):
-            since_factor = max(REFACTOR_EVERY, 2 * m)       # the two ways to the pivot element disagree
-            continue
         target = lo[head[r]] if below else hi[head[r]]
         theta_p = (xB[r] - target) / alpha_q[r]
         xB = xB - theta_p * alpha_q
@@ -335,4 +347,4 @@ def dual_simplex(A, b, c, l, u, row_on=None, col_status=None, row_status=None,
         obj = obj + cost[j] * x_all[j]
     return SimplexResult(status=status, objective=float(obj), x=x_all[:n].copy(), y=y.copy(), rc=d[:n].copy(),
                          col_status=stat[:n].copy(), row_status=stat[n:].copy(), pivots=pivots,
-                         head=head.copy(), Binv=Binv, flips=flips_total, weights=w.copy())
+                         head=head.copy(), Binv=Binv, flips=flips_total, weights=w.copy(), refused=refused)

@@ -1520,6 +1520,10 @@ int sx_run(blp_handle h, int B, const SxStage& S, bool use_parent, int max_pivot
     SxBatch Q{};
     Q.B = B;
     Q.max_pivots = max_pivots;
+    // test knobs of a tuning build: a negative mismatch threshold refuses every pivot that does not directly
+    // follow a factorisation, a small interval forces the periodic refactorisation
+    Q.pivot_mismatch = env_dbl("BLP_SX_MISMATCH", kSxPivotMismatch);
+    Q.refactor_every = env_int("BLP_SX_REFACTOR_EVERY", 0);
     Q.lb = S.lb; Q.ub = S.ub; Q.rowon = S.mask; Q.cstat_in = S.cs; Q.rstat_in = S.rs;
     Q.parent = use_parent ? S.parent : nullptr;
     Q.Binv = h->sx_binv[cur].as<double>(); Q.head = h->sx_head[cur].as<int32_t>();

@@ -43,6 +43,8 @@ struct SxProb {
 // per-call arrays; node k uses slice k of each
 struct SxBatch {
     int B, max_pivots;
+    double pivot_mismatch;                     // kSxPivotMismatch (a tuning build reads BLP_SX_MISMATCH)
+    int refactor_every;                        // 0: max(kSxRefactorEvery, 2 m) (BLP_SX_REFACTOR_EVERY)
     const double* lb; const double* ub;        // [B][n] node major
     const uint8_t* rowon;                      // [B][m - m_base] or null (all pool rows on)
     const int8_t* cstat_in; const int8_t* rstat_in;   // [B][n], [B][m] CLP codes, or null = slack basis
@@ -588,7 +590,7 @@ __device__ void sx_solve_node(const SxProb& P, const SxBatch& Q, const int node,
     int pivots = 0, flips_total = 0, since_factor = 0, status = 0;
     // no anti-cycling rule: a hard cap far above any pivot count seen ends a cycling node with status 3
     const int pivot_cap = min(Q.max_pivots, 50 * N + 1000);
-    const int refactor_every = max(kSxRefactorEvery, 2 * m);
+    const int refactor_every = Q.refactor_every > 0 ? Q.refactor_every : max(kSxRefactorEvery, 2 * m);
     auto score_of = [&](const int i) {
         const int hv = nd.head[i];
         const double xb = nd.xB[i];
@@ -708,8 +710,19 @@ __device__ void sx_solve_node(const SxProb& P, const SxBatch& Q, const int node,
         const int q = C.q;
         if (q < 0) { status = 1; break; }
         const int nflip = C.nflip;
+        // ---- entering column; the mismatch check comes before anything of the pivot is applied -------
+        sx_ftran_col(T, P, nd, q, nd.aq);
+        T.sync();                                          // barrier 2: alpha_q complete, every CTA has set its flip marks
+        const double piv = nd.aq[r];
+        if (since_factor > 0 && fabs(sx_sub(piv, nd.ar[q])) > sx_mul(Q.pivot_mismatch, sx_add(1.0, fabs(nd.ar[q])))) {
+            // the two ways to the pivot element disagree: refactorise and price again with nothing applied.
+            // Flipping first would leave the flipped columns on the bound their reduced costs say is wrong.
+            if (nflip > 0)
+                for (int j = T.tid; j < N; j += T.nth) nd.flip[j] = 0;   // read again after the refactorisation's barriers
+            since_factor = refactor_every;
+            continue;
+        }
         if (nflip > 0) {
-            T.sync();                                      // every CTA has set its marks before they are cleared
             // xfull <- bound moves of the flipped columns; col = A delta - delta_slack; x_B -= Binv col
             for (int j = T.tid; j < N; j += T.nth) {
                 double dl = 0.0;
@@ -728,18 +741,12 @@ __device__ void sx_solve_node(const SxProb& P, const SxBatch& Q, const int node,
                 nd.col[i] = sx_sub(acc, nd.xfull[n + i]);
             }
             T.sync();
-            sx_matvec(T, nd, nd.col, nd.aq);               // thread i writes aq[i] and is the one to use it
-            for (int i = T.tid; i < m; i += T.nth) nd.xB[i] = sx_sub(nd.xB[i], nd.aq[i]);
+            sx_matvec(T, nd, nd.col, nd.rho);              // rho is free until the pivot row is staged below;
+            for (int i = T.tid; i < m; i += T.nth) nd.xB[i] = sx_sub(nd.xB[i], nd.rho[i]);   // thread i wrote rho[i]
+            T.sync();                                      // the flipped x_B complete
             flips_total += nflip;
         }
-        // ---- entering column, step lengths, updates -----------------------------------------------
-        sx_ftran_col(T, P, nd, q, nd.aq);
-        T.sync();                                          // barrier 2: alpha_q (and the flipped x_B) complete
-        const double piv = nd.aq[r];
-        if (since_factor > 0 && fabs(sx_sub(piv, nd.ar[q])) > sx_mul(kSxPivotMismatch, sx_add(1.0, fabs(nd.ar[q])))) {
-            since_factor = refactor_every;                // the two ways to the pivot element disagree
-            continue;
-        }
+        // ---- step lengths, updates ----------------------------------------------------------------
         const double target = below ? nd.lo[leaving] : nd.hi[leaving];
         const double theta_p = sx_sub(nd.xB[r], target) / piv;
         const double xq_new = sx_add(nd.stat[q] == SX_UPPER ? nd.hi[q] : nd.lo[q], theta_p);
