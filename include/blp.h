@@ -200,8 +200,8 @@ int blp_solve_children_host(blp_handle h, int B, const double* parent_lb, const 
 
 /*
  * Dual simplex path for small and mid-size node LPs (at most blp_simplex_max_rows() rows incl. appended cut
- * rows): one CTA per node — for LPs of more than blp_simplex_batch_rows() rows the whole GPU, cooperatively, one
- * node after the other — runs a bounded dual simplex with a dense basis inverse (dual steepest edge pricing,
+ * rows): one CTA per node — for LPs of more than blp_simplex_batch_rows() rows a group of SMs per node, the
+ * groups side by side in one cooperative launch, each through its share of the batch — runs a bounded dual simplex with a dense basis inverse (dual steepest edge pricing,
  * bound flipping ratio test; csrc/blp_simplex.cuh, restated in numpy in oracle/dual_simplex.py). It
  * returns what the reference reads from CLP after lp.dual(): a VERTEX and its BASIS, so that the
  * integrality test (base_node.py:281-283), the most fractional index (:544-562), the tableau
@@ -222,8 +222,8 @@ int blp_solve_children_host(blp_handle h, int B, const double* parent_lb, const 
  * stats (may be NULL): iterations = max pivots of a node, node_iterations = sum of pivots, total_ms,
  * step_kernel_ms = the simplex kernel, kernel_launches, refills = bound flips of the ratio tests.
  */
-int blp_simplex_max_rows(void);        /* 8192: above blp_simplex_batch_rows() the whole GPU works on one node at a time */
-int blp_simplex_batch_rows(void);      /* 1024: up to here one CTA per node, the batch is one launch */
+int blp_simplex_max_rows(void);        /* 8192: above blp_simplex_batch_rows() a group of SMs works on each node */
+int blp_simplex_batch_rows(void);      /* 1024: up to here one CTA per node */
 int blp_simplex_batch_host(blp_handle h, int B, const double* lb, const double* ub, const uint8_t* row_mask,
                            const int8_t* col_status, const int8_t* row_status, const int32_t* parent_slot,
                            int max_pivots, double* obj, int32_t* status, int32_t* pivots, double* x,

@@ -31,7 +31,8 @@ COIN_INFINITY = 1.7976931348623157e308      # what CyClpSimplex.getCoinInfinity(
 # pivots, base_node.py:645; a first-order iteration is far cheaper than a pivot)
 PDHG_ITERS_PER_PIVOT = 512
 
-# device memory the dense basis inverses of one simplex call may take ('auto' method selection)
+# device memory the dense basis inverses of one simplex call may take: 'auto' sends a larger batch to PDHG,
+# 'simplex' splits it into consecutive calls
 SIMPLEX_MEMORY_BUDGET = 16 << 30
 SIMPLEX_WIDE_MAX_BATCH = 2
 
@@ -240,13 +241,18 @@ class SharedLP:
         if ok and self.method == 'auto':
             m = self.m + len(self.cut_rows)
             ok = n_lps * m * m * 8 <= SIMPLEX_MEMORY_BUDGET
-            # mid-size LPs (the whole GPU per node, one after the other): only where the vertex is what
-            # the caller is after — a single node's bound / cut round; batches go to PDHG
+            # mid-size LPs (a group of SMs per node): only where the vertex is what the caller is after —
+            # a single node's bound / cut round; batches go to PDHG
             if ok and not getattr(eng, 'simplex_batched', True):
                 ok = n_lps <= SIMPLEX_WIDE_MAX_BATCH
         if not ok and self.method == 'simplex':
             raise RuntimeError('the LP is too large for the dual simplex path')
         return ok
+
+    def simplex_call_size(self, n_lps: int) -> int:
+        """LPs per simplex call: as many as SIMPLEX_MEMORY_BUDGET holds dense basis inverses of, at least one."""
+        m = self.m + len(self.cut_rows)
+        return max(1, min(n_lps, SIMPLEX_MEMORY_BUDGET // (m * m * 8)))
 
     def sync_cuts(self):
         if self._on_device < len(self.cut_rows):
@@ -759,7 +765,10 @@ def _solve_group(sh: SharedLP, batch: List[CyClpSimplex], budget: int, default_o
             sh.register_cut(lp._cut_keys[nm], pi, pi0)
     sh.sync_cuts()
     if sh.use_simplex(len(batch)):
-        _solve_group_simplex(sh, batch, budget, default_opts)
+        # a later call starts its LPs from their basis status: the store holds the factors of the last call only
+        step = sh.simplex_call_size(len(batch))
+        for k0 in range(0, len(batch), step):
+            _solve_group_simplex(sh, batch[k0:k0 + step], budget, default_opts)
     else:
         _solve_group_pdhg(sh, batch, budget, default_opts)
     for lp in batch:

@@ -1501,6 +1501,16 @@ int sx_carve(blp_handle h, int B, bool want_mask, bool want_status, bool want_pa
     return BLP_OK;
 }
 
+// Groups of SMs that k_simplex_wide runs side by side for a batch of B mid-size LPs of m rows: G = min(B,
+// Gmax(m)), S = SMs / G CTAs per group. A group's pivot is bound by its barriers and by the rows every CTA
+// scans for its own decisions, not by bandwidth, so small LPs gain from many groups and large ones, whose
+// inverses compete for HBM, from few. Gmax(m) is fitted from the sweep of tools/gpu_simplex_groups.py
+// (profiles/simplex_groups_sweep.json, DESIGN section 2b).
+int sx_groups(int m, int B) {
+    const int gmax = m <= 5000 ? 64 : 16;
+    return std::min(B, gmax);
+}
+
 // launch the simplex kernel on staged inputs, copy the results back to the host
 int sx_run(blp_handle h, int B, const SxStage& S, bool use_parent, int max_pivots, double* obj,
            int32_t* status, int32_t* pivots, double* x, double* y, double* rc, int8_t* cso, int8_t* rso,
@@ -1538,19 +1548,20 @@ int sx_run(blp_handle h, int B, const SxStage& S, bool use_parent, int max_pivot
         const int threads = m <= 128 ? 128 : 512;
         k_simplex<<<B, threads, 0, st>>>(P, Q);
     } else {
-        // the whole GPU on one node at a time: cooperative grid, one CTA per SM
+        // one cooperative grid, one CTA per SM, split into G groups of S CTAs; group g solves nodes g, g + G, ...
         if (!h->coop_ok) return fail(BLP_ERR_STATE, "blp_simplex: LPs of more than %d rows need cooperative launches", kSxMaxRows);
         int occ = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_simplex_wide, 512, 0));
         if (occ < 1) return fail(BLP_ERR_STATE, "blp_simplex: k_simplex_wide does not fit an SM");
-        const int grid = h->num_sms;
-        CK(h->sx_wide.ensure(256));
-        unsigned* counter = h->sx_wide.as<unsigned>();
-        for (int node = 0; node < B; ++node) {
-            CK(cudaMemsetAsync(counter, 0, sizeof(unsigned), st));      // the grid barrier's arrival counter
-            void* args[] = {(void*)&P, (void*)&Q, (void*)&node, (void*)&counter};
-            CK(cudaLaunchCooperativeKernel((const void*)k_simplex_wide, dim3(grid), dim3(512), args, 0, st));
-        }
+        // a tuning build forces G through BLP_SX_GROUPS, clamped to [1, min(B, SMs)]
+        const int G = std::max(1, std::min(env_int("BLP_SX_GROUPS", sx_groups(m, B)), std::min(B, h->num_sms)));
+        const int grid = G * (h->num_sms / G);
+        if (grid > occ * h->num_sms) return fail(BLP_ERR_STATE, "blp_simplex: %d CTAs are not co-resident", grid);
+        CK(h->sx_wide.ensure((size_t)G * kSxBarrierStride * sizeof(unsigned)));
+        unsigned* counters = h->sx_wide.as<unsigned>();
+        CK(cudaMemsetAsync(counters, 0, (size_t)G * kSxBarrierStride * sizeof(unsigned), st));  // the groups' arrival counters
+        void* args[] = {(void*)&P, (void*)&Q, (void*)&G, (void*)&counters};
+        CK(cudaLaunchCooperativeKernel((const void*)k_simplex_wide, dim3(grid), dim3(512), args, 0, st));
     }
     CK(cudaGetLastError());
     CK(cudaEventRecord(h->ev[3], st));

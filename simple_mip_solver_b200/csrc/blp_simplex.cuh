@@ -24,7 +24,7 @@
 namespace blp {
 
 constexpr int kSxMaxRows = 1024;          // one CTA per node (k_simplex)
-constexpr int kSxMaxRowsWide = 8192;      // the whole GPU per node (k_simplex_wide, cooperative launch)
+constexpr int kSxMaxRowsWide = 8192;      // a group of SMs per node (k_simplex_wide, cooperative launch)
 constexpr int kSxWeightLanes = 16;
 constexpr int SX_BASIC = 1, SX_UPPER = 2, SX_LOWER = 3;
 constexpr double kSxPrimalTol = 1e-9, kSxDualTol = 1e-9, kSxPivTol = 1e-9, kSxTieRel = 1e-12;
@@ -153,16 +153,22 @@ __device__ __forceinline__ SxCand sx_block_best(SxCand c, SxCandRed& s) {
 }
 
 
-// ---- the team that works on ONE node: a CTA (k_simplex) or the whole cooperative grid (k_simplex_wide) ----
+// ---- the team that works on ONE node: a CTA (k_simplex) or a group of CTAs of the cooperative grid (k_simplex_wide) ----
 // Array work (the O(m^2) sweep, row / column dots, vector updates) is split over the team's threads and
 // followed by a team barrier. DECISIONS (pricing, ratio test, pivot row of a factorisation step) are
 // taken by every CTA for itself from the shared arrays: the reductions are max / min / lexicographic min
 // over all m or n+m elements — cheap, order independent, so every CTA reaches the same decision and the
-// scalars live in its own shared memory; no cross-CTA reduction, no barrier per decision. A grid team
+// scalars live in its own shared memory; no cross-CTA reduction, no barrier per decision. A group team
 // therefore needs 5 barriers per pivot (8 with bound flips) and both teams compute bit-identical results.
 struct SxCtrl {            // per-CTA scalars: one thread decides, the CTA reads them after __syncthreads
     int r, q, nflip, status, par_ok;
     double slope;
+};
+
+struct SxGroupBar {        // per-CTA view of its group's barrier (shared memory)
+    unsigned* counter;     // the group's arrival counter (zeroed before the launch)
+    unsigned gen;          // this CTA's barrier generation; carries over from one node of the group to the next
+    unsigned nctas;        // CTAs of the group
 };
 
 template <bool WIDE>
@@ -171,22 +177,21 @@ struct SxTeam {
     SxRed* red;            // shared memory of this CTA
     SxCandRed* cred;
     SxCtrl* ctrl;
-    unsigned* bar;         // grid team: arrival counter of the barrier (zeroed before the launch)
-    unsigned* gen;         // ... and this CTA's barrier generation (shared memory)
+    SxGroupBar* bar;       // group team only
 
-    // Barrier over the team. Grid team: every CTA arrives once per generation on a global counter; thread 0
-    // spins until all have (the cooperative launch guarantees co-residency). The gpu-scope fences order
-    // the CTA's earlier global writes before the arrival and drop its stale L1 lines after it.
+    // Barrier over the team. Group team: every CTA of the group arrives once per generation on the group's
+    // counter; thread 0 spins until all have (the cooperative launch guarantees co-residency). The gpu-scope
+    // fences order the CTA's earlier global writes before the arrival and drop its stale L1 lines after it.
     __device__ __forceinline__ void sync() const {
         if (!WIDE) { __syncthreads(); return; }
         __syncthreads();
         if (threadIdx.x == 0) {
-            const unsigned target = (*gen + 1u) * gridDim.x;
+            const unsigned target = (bar->gen + 1u) * bar->nctas;
             __threadfence();
-            atomicAdd(bar, 1u);
-            while (*reinterpret_cast<volatile unsigned*>(bar) < target) __nanosleep(32);
+            atomicAdd(bar->counter, 1u);
+            while (*reinterpret_cast<volatile unsigned*>(bar->counter) < target) __nanosleep(32);
             __threadfence();
-            *gen += 1u;
+            bar->gen += 1u;
         }
         __syncthreads();
     }
@@ -839,25 +844,33 @@ k_simplex(const SxProb P, const SxBatch Q) {
     SxTeam<false> T;
     T.tid = threadIdx.x; T.nth = blockDim.x; T.lane = threadIdx.x & 31; T.warp = threadIdx.x >> 5;
     T.nwarps = blockDim.x >> 5;
-    T.red = &red; T.cred = &cred; T.ctrl = &ctrl; T.bar = nullptr; T.gen = nullptr;
+    T.red = &red; T.cred = &cred; T.ctrl = &ctrl; T.bar = nullptr;
     sx_solve_node<false>(P, Q, blockIdx.x, T);
 }
 
-// The whole GPU on ONE node (cooperative launch, one CTA per SM): LPs of up to kSxMaxRowsWide rows, whose
-// dense inverse (m^2 doubles: 200 MB at m = 5000) is swept by all SMs at once. Same code, same results.
+// G groups of S CTAs in one cooperative launch (one CTA per SM, grid = G S): LPs of up to kSxMaxRowsWide rows,
+// whose dense inverse (m^2 doubles: 200 MB at m = 5000) is swept by the S SMs of a group at once. Group g
+// solves nodes g, g + G, g + 2G, ... one after the other; G = 1 is the whole GPU on each node. Same code,
+// same results. Each group's arrival counter sits on its own 128-byte line (kSxBarrierStride unsigneds).
+constexpr int kSxBarrierStride = 32;
 __global__ void __launch_bounds__(512, 1)
-k_simplex_wide(const SxProb P, const SxBatch Q, const int node, unsigned* const barrier_counter) {
+k_simplex_wide(const SxProb P, const SxBatch Q, const int groups, unsigned* const barrier_counters) {
     __shared__ SxRed red;
     __shared__ SxCandRed cred;
     __shared__ SxCtrl ctrl;
-    __shared__ unsigned gen;
-    if (threadIdx.x == 0) gen = 0u;
+    __shared__ SxGroupBar bar;
+    const int S = gridDim.x / groups, g = blockIdx.x / S;
+    if (threadIdx.x == 0) {
+        bar.counter = barrier_counters + (size_t)g * kSxBarrierStride;
+        bar.gen = 0u;
+        bar.nctas = (unsigned)S;
+    }
     __syncthreads();
     SxTeam<true> T;
-    T.tid = blockIdx.x * blockDim.x + threadIdx.x; T.nth = gridDim.x * blockDim.x; T.lane = threadIdx.x & 31;
+    T.tid = (blockIdx.x % S) * blockDim.x + threadIdx.x; T.nth = S * blockDim.x; T.lane = threadIdx.x & 31;
     T.warp = T.tid >> 5; T.nwarps = T.nth >> 5;
-    T.red = &red; T.cred = &cred; T.ctrl = &ctrl; T.bar = barrier_counter; T.gen = &gen;
-    sx_solve_node<true>(P, Q, node, T);
+    T.red = &red; T.cred = &cred; T.ctrl = &ctrl; T.bar = &bar;
+    for (int node = g; node < Q.B; node += groups) sx_solve_node<true>(P, Q, node, T);
 }
 
 // Rows of the simplex tableau Binv [A, -I] of a node whose factor is in a store (device-side GMI

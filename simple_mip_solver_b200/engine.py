@@ -325,8 +325,9 @@ class BatchLP:
 
     @property
     def simplex_batched(self) -> bool:
-        """True when a simplex batch is ONE launch (one CTA per node); beyond blp_simplex_batch_rows()
-        rows the whole GPU works on one node at a time."""
+        """True when a simplex batch runs one CTA per node; beyond blp_simplex_batch_rows() rows a group
+        of SMs works on each node (one cooperative launch, the groups side by side, each through its share of
+        the batch), so a batch takes longer per node and a whole strong-branching round may not fit in memory."""
         return self.m <= self._lib.blp_simplex_batch_rows()
 
     def _simplex_out(self, B, m):
