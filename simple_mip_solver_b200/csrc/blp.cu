@@ -743,11 +743,12 @@ int blp_create(int device, int m, int n, int64_t nnz, const int32_t* rowptr, con
     cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, device);
     cudaDeviceGetAttribute(&h->coop_ok, cudaDevAttrCooperativeLaunch, device);
     cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
-    // the wide step kernels carry ~8 KB of static shared memory next to a slab of up to 44 KB: opt in above 48 KB
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_primal2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_primal2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_dual2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_dual2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+    // the wide step kernels carry ~8 KB of static shared memory next to a slab of up to 44 KB and the scalars of up
+    // to kMaxChunkRows rows (24 KB): opt in above 48 KB
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_primal2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_primal2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_dual2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_dual2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024);
     if (e == cudaSuccess) e = cudaMallocHost(&h->h_counters, 16 * sizeof(int32_t));
     for (int q = 0; q < 4 && e == cudaSuccess; ++q) e = cudaEventCreate(&h->ev[q]);
     for (int q = 0; q < blp_handle_s::kLanes - 1 && e == cudaSuccess; ++q) {
@@ -936,7 +937,9 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
     auto step_plan = [&](int rows, int width, bool primal = false) {
         // two nodes per lane pay off when a launch has real work; tiny LPs stay on the
         // one-node-per-lane kernels, which can run a whole period as one cooperative launch
-        const bool v2 = allow_v2 && width >= kBlk && (long)std::max(P.n, P.m) * width >= (1L << 20);
+        // (k_primal2 / k_dual2 index the state with 32 bits)
+        const bool v2 = allow_v2 && width >= kBlk && (long)std::max(P.n, P.m) * width >= (1L << 20) &&
+                        (size_t)std::max(P.n, P.m) * S.ld < ((size_t)1 << 32);
         int r = v2 ? (primal ? rpw2p : rpw2) : rpw;
         Plan p = make_plan(rows, width, r, 0);
         auto shape = [&](Plan& q, int rr) {
@@ -958,6 +961,10 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
     auto finish_step_plans = [&]() -> int {
         plan_chunks(pc, h->hptrAT, P.n, h->h_chunkC);
         plan_chunks(pr, h->hptrA, P.m, h->h_chunkR);
+        if (pc.V == 2) {                           // k_primal2 / k_dual2 stage their rows' scalars behind the slab
+            pc.smem += (size_t)kPrimalRowBytes * pc.rows_per_cta;
+            pr.smem += (size_t)kDualRowBytes * pr.rows_per_cta;
+        }
         CK(upload(h->chunkC, h->h_chunkC, st));
         CK(upload(h->chunkR, h->h_chunkR, st));
         pc.chunk_ptr = h->chunkC.as<int32_t>();

@@ -227,14 +227,24 @@ struct Slab {
 
 extern __shared__ int4 dyn_smem[];
 
+// Per-row scalars a slab stage can copy to shared memory along with the row pointers: rs(j, slot) loads
+// those of global row j and stores them at `slot` (the row's place in the CTA's work list).
+struct NoRowScalars {
+    __device__ __forceinline__ void operator()(int, int) const {}
+};
+
+template <class RS = NoRowScalars>
 __device__ __forceinline__ Slab stage_slab(const int32_t* __restrict__ ptr,
                                            const Ent* __restrict__ ent, const int r0, const int r1,
                                            const int rows_per_cta, const int cap,
-                                           int4* const smem_base = dyn_smem) {
+                                           int4* const smem_base = dyn_smem, const RS rs = RS()) {
     int* sp = reinterpret_cast<int*>(smem_base);
     int4* se = smem_base + (rows_per_cta + 4) / 4;
     const int nrows = r1 - r0;
-    for (int t = threadIdx.x; t <= nrows; t += kCtaThreads) sp[t] = __ldg(ptr + r0 + t);
+    for (int t = threadIdx.x; t <= nrows; t += kCtaThreads) {
+        sp[t] = __ldg(ptr + r0 + t);
+        if (t < nrows) rs(r0 + t, t);
+    }
     __syncthreads();
     Slab s;
     s.sp = sp;
@@ -530,20 +540,24 @@ __device__ __forceinline__ void st2(double* p, const double2 v, const bool k0, c
 }
 
 // ld: distance (in doubles) between consecutive rows of the gathered vector (kBlk for the solver's
-// tile-major state, the caller's leading dimension for blp_spmv)
-template <bool SHARED>
+// tile-major state, the caller's leading dimension for blp_spmv). Row col of the lane's column is at
+// Vn + off + col * ld, computed in the index type I (the step kernels use 32 bits, see k_primal2).
+// PAD = false leaves the slots of a batch past the row's end unset (they are never read): at 48 registers that
+// is what lets the step kernels keep a full batch of gathers in flight (k_spmv2 spills without the padding).
+template <bool SHARED, class I = size_t, bool PAD = true>
 __device__ __forceinline__ void dot2_entries(const int4* __restrict__ E, const int p0, const int p1,
                                              const double* __restrict__ Vn, double& g0, double& g1,
-                                             const int ld = kBlk) {
+                                             const int ld = kBlk, const I off = 0) {
     constexpr int kU = BLP_U;
+#pragma unroll 1
     for (int p = p0; p < p1; p += kU) {
         double2 v[kU];
 #pragma unroll
         for (int q = 0; q < kU; ++q) {
-            v[q] = make_double2(0.0, 0.0);
+            if (PAD) v[q] = make_double2(0.0, 0.0);
             if (p + q < p1) {
                 const int col = SHARED ? E[p + q].x : __ldg(&E[p + q].x);
-                v[q] = ld2(Vn + (size_t)col * ld);
+                v[q] = ld2(Vn + (off + (I)col * (I)ld));
             }
         }
 #pragma unroll
@@ -660,11 +674,13 @@ __shared__ int s_nrows;
 // everything), compacted so the warps share them evenly — and the ends of the rows' kept entries in the tile's
 // folded matrix `ent`. Everything global is loaded in the two phases stage_slab has anyway (pointers, ends and
 // flags together, then the entries), so a CTA pays no extra round trip. `live`: the warp's ballot of running lanes,
-// lanes 0-15 hold the nodes of block h0, lanes 16-31 those of h0 + 1.
+// lanes 0-15 hold the nodes of block h0, lanes 16-31 those of h0 + 1. `rs`: per-row scalars of the work-list rows,
+// loaded in phase 2 with the entries.
+template <class RS>
 __device__ __forceinline__ Slab stage_slab_frozen(const int32_t* __restrict__ ptr, const Ent* __restrict__ ent,
                                                   const int32_t* __restrict__ ends, const uint8_t* __restrict__ flags,
                                                   const int rows, const int h0, const unsigned live, const int r0,
-                                                  const int r1, const int rows_per_cta, const int cap) {
+                                                  const int r1, const int rows_per_cta, const int cap, const RS rs) {
     int* sp = reinterpret_cast<int*>(dyn_smem);
     int4* se = dyn_smem + (rows_per_cta + 4) / 4;
     const int nrows = r1 - r0, lane = threadIdx.x & 31;
@@ -708,6 +724,7 @@ __device__ __forceinline__ Slab stage_slab_frozen(const int32_t* __restrict__ pt
             int before = 0;
             for (int g = 0; g < (t >> 5); ++g) before += s_group[g];
             s_rows[before + rank[q]] = (uint16_t)t;
+            rs(r0 + t, before + rank[q]);
         }
     }
     if (threadIdx.x == 0) {
@@ -729,6 +746,68 @@ __device__ __forceinline__ Slab stage_slab_frozen(const int32_t* __restrict__ pt
 #define BLP_MINB2P 4          // resident CTAs per SM the paired primal kernel is compiled for
 #endif
 
+// What a warp's trip over one row reads besides the row's state and gathers, staged with the slab (no round trip of
+// its own) and read from shared memory after the gathers are issued. At 48 registers (5 CTAs per SM) the compiler
+// can only keep a full BLP_U batch of gathers in flight when nothing else is live across them: with these scalars
+// loaded from global memory inside the trip it issued one gather at a time in the primal step and two in the dual
+// step, and the trip waited on the bound mask before its first gather (DESIGN §4).
+// Per-lane loop invariants of the two-nodes-per-lane steps: (w0, w1) and (tau0, tau1) / (sigma0, sigma1).
+__shared__ double2 s_wv[32], s_sv[32];
+
+// Dynamic shared memory behind a step kernel's slab (row pointers, `cap` entries) that holds its row scalars.
+__device__ __forceinline__ int4* row_scalar_smem(const int rows_per_cta, const int cap) {
+    return dyn_smem + (rows_per_cta + 4) / 4 + cap;
+}
+// Bytes per chunk row (host side sizes the launch with them).
+constexpr int kPrimalRowBytes = 48, kDualRowBytes = 16;
+
+// primal step: c_j, and (lref, uref), lumask of row j in the tile's two 32-node blocks h0, h0 + 1
+struct PrimalRowScalars {
+    const double* c; const double* lref; const double* uref; const uint32_t* lumask;   // at block h0
+    size_t rows;                                                                    // block stride
+    // the staged arrays; a trip rebuilds this from the kernel parameters instead of keeping pointers in registers
+    struct View {
+        double2* lu; double* cs; uint32_t* mk;                                      // [slot][2], [slot], [slot][2]
+        __device__ __forceinline__ View(const int rows_per_cta, const int cap) {
+            lu = reinterpret_cast<double2*>(row_scalar_smem(rows_per_cta, cap));
+            cs = reinterpret_cast<double*>(lu + 2 * rows_per_cta);
+            mk = reinterpret_cast<uint32_t*>(cs + rows_per_cta);
+        }
+    };
+    View v;
+    __device__ PrimalRowScalars(const DevProb& P, const DevState& S, const int h0, const int rows_per_cta,
+                                const int cap) : v(rows_per_cta, cap) {
+        const size_t f = (size_t)h0 * P.n;
+        c = P.c; lref = S.lref + f; uref = S.uref + f; lumask = S.lumask + f; rows = P.n;
+    }
+    __device__ __forceinline__ void operator()(const int j, const int slot) const {
+        v.cs[slot] = __ldg(c + j);
+        v.lu[2 * slot] = make_double2(__ldg(lref + j), __ldg(uref + j));
+        v.lu[2 * slot + 1] = make_double2(__ldg(lref + rows + j), __ldg(uref + rows + j));
+        v.mk[2 * slot] = __ldg(lumask + j);
+        v.mk[2 * slot + 1] = __ldg(lumask + rows + j);
+    }
+};
+
+// dual step: b_i, and rconst of row i in the tile (frozen coordinates) or 0
+struct DualRowScalars {
+    const double* b; const double* rc;      // rc: null without frozen coordinates
+    struct View {
+        double* bs; double* rcs;            // [slot], [slot]
+        __device__ __forceinline__ View(const int rows_per_cta, const int cap) {
+            bs = reinterpret_cast<double*>(row_scalar_smem(rows_per_cta, cap));
+            rcs = bs + rows_per_cta;
+        }
+    };
+    View v;
+    __device__ DualRowScalars(const DevProb& P, const double* rconst, const int rows_per_cta, const int cap)
+        : b(P.b), rc(rconst), v(rows_per_cta, cap) {}
+    __device__ __forceinline__ void operator()(const int i, const int slot) const {
+        v.bs[slot] = __ldg(b + i);
+        v.rcs[slot] = rc ? __ldg(rc + i) : 0.0;
+    }
+};
+
 template <bool MAJOR>
 __global__ void __launch_bounds__(kCtaThreads, BLP_PAIR_ROWS ? BLP_MINB2P : BLP_MINB2)
 k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_cta, const int cap,
@@ -739,6 +818,11 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
     const bool k1 = node + 1 < S.B && S.fin[node + 1] == 0;
     const unsigned live = __ballot_sync(0xffffffffu, k0 || k1);
     if (live == 0) return;                                     // whole block retired
+    // which lanes store node / node + 1: warp-uniform masks, so that the trip keeps no predicate registers for them
+    // (the gather batch needs them). The MAJOR step keeps k0 / k1: with the masks it spills.
+    const unsigned run0 = __ballot_sync(0xffffffffu, k0), run1 = __ballot_sync(0xffffffffu, k1);
+    auto st0 = [&] { return MAJOR ? k0 : ((run0 >> (threadIdx.x & 31)) & 1u) != 0; };
+    auto st1 = [&] { return MAJOR ? k1 : ((run1 >> (threadIdx.x & 31)) & 1u) != 0; };
     double w0 = 0, w1 = 0, tau0 = 0, tau1 = 0;
     if (k0) {
         const int s = S.sbase[node] + it;
@@ -750,19 +834,29 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
         w1 = (double)s / (double)(s + 1);
         tau1 = S.eta[node + 1] / S.omega[node + 1];
     }
+    if (warp == 0) {                                           // every warp has the same; read back after the stage
+        s_wv[lane] = make_double2(w0, w1);
+        s_sv[lane] = make_double2(tau0, tau1);
+    }
     const int r0 = __ldg(chunk_ptr + 2 * blockIdx.x);
     const int r1 = __ldg(chunk_ptr + 2 * blockIdx.x + 1);
     const bool frz = !MAJOR && S.cfrz != nullptr;
     const int tile = tile0 + blockIdx.y;
     // with frozen coordinates: the tile's folded A' (entries of frozen rows, whose multiplier is zero, taken out)
     const Ent* __restrict__ cent = frz ? S.fentAT + (size_t)tile * P.nnz : P.cent;
+    const PrimalRowScalars rs(P, S, tile * 2, rows_per_cta, cap);
     const Slab sl = frz ? stage_slab_frozen(P.cptr, cent, S.fendAT + (size_t)tile * P.n, S.cfrz, P.n, tile * 2, live,
-                                            r0, r1, rows_per_cta, cap)
-                        : stage_slab(P.cptr, P.cent, r0, r1, rows_per_cta, cap);
-    const size_t base = tix(0, node, P.n);
+                                            r0, r1, rows_per_cta, cap, rs)
+                        : stage_slab(P.cptr, P.cent, r0, r1, rows_per_cta, cap, dyn_smem, rs);
+    // 32-bit element indices: the host picks these kernels only for state arrays of fewer than 2^32 elements
+    const unsigned base = (unsigned)tix(0, node, P.n);
     const double* __restrict__ yn = S.y + tix(0, node, P.m);
+    const unsigned yoff = (unsigned)tix(0, node, P.m);
+#if BLP_PAIR_ROWS
     const size_t fblk = (size_t)(node >> 5) * P.n;
+#endif
     const unsigned bit = node & 31;
+    const int half = lane >> 4;                                // lanes 16-31: nodes of block h0 + 1
     const bool coop = (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
     double cg0 = 0.0, cg1 = 0.0;
     if (coop) {
@@ -831,32 +925,58 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
         return;
     }
 #endif
-    const int ntrips = frz ? s_nrows : r1 - r0;                // frozen columns rest at their bound for the whole tile
-    for (int k = warp; k < ntrips; k += kWarps) {
-        const int j = r0 + (frz ? (int)s_rows[k] : k);
-        const size_t e = base + (size_t)j * kBlk;
+    // one warp trip: row slot k of the work list; gather(lr, g0, g1) adds the row's gather-dot to (g0, g1)
+    auto trip = [&](const int k, double g0, double g1, auto gather) {
+        const int lr = frz ? (int)s_rows[k] : k;
+        const unsigned e = base + (unsigned)(r0 + lr) * kBlk;
         const double2 xb = ld2(S.xbar + e);
         const double2 a = ldcs2(S.xa + e);
-        const uint32_t mk = (__ldg(S.lumask + fblk + j) >> bit) & 3u;
-        double lo0 = __ldg(S.lref + fblk + j), hi0 = __ldg(S.uref + fblk + j);
-        double lo1 = lo0, hi1 = hi0;
-        if (mk) {                                              // a node of this lane deviates
-            const double2 l2 = ldcs2(S.l + e), u2 = ldcs2(S.u + e);
-            if (mk & 1u) { lo0 = l2.x; hi0 = u2.x; }
-            if (mk & 2u) { lo1 = l2.y; hi1 = u2.y; }
+        gather(lr, g0, g1);
+        // the rest of the row's inputs come from shared memory once the gathers fly; the dense bounds of nodes
+        // that deviate from their block's reference (about 1 % of rows) only after them
+        const PrimalRowScalars::View rv(rows_per_cta, cap);
+        const uint32_t mk = (rv.mk[2 * k + half] >> bit) & 3u;
+        const double2 lh = rv.lu[2 * k + half];
+        double lo0 = lh.x, hi0 = lh.y, lo1 = lh.x, hi1 = lh.y;
+        if (mk & 1u) {                                         // node deviates from its block's reference
+            lo0 = __ldcs(S.l + e);
+            hi0 = __ldcs(S.u + e);
         }
-        double g0 = cg0, g1 = cg1;
-        if (!coop) slab_dot2(sl, cent, j - r0, yn, g0, g1);
-        const double cj = __ldg(P.c + j);
-        const double xc0 = fma(w0, xb.x - a.x, a.x), xc1 = fma(w1, xb.y - a.y, a.y);
-        const double xp0 = fmin(fmax(xc0 - tau0 * (cj - g0), lo0), hi0);
-        const double xp1 = fmin(fmax(xc1 - tau1 * (cj - g1), lo1), hi1);
-        st2(S.xbar + e, make_double2(2.0 * xp0 - xc0, 2.0 * xp1 - xc1), k0, k1);
+        if (mk & 2u) {
+            lo1 = __ldcs(S.l + e + 1);
+            hi1 = __ldcs(S.u + e + 1);
+        }
+        const double cj = rv.cs[k];
+        const double2 w = s_wv[lane], tau = s_sv[lane];
+        const double xc0 = fma(w.x, xb.x - a.x, a.x), xc1 = fma(w.y, xb.y - a.y, a.y);
+        const double xp0 = fmin(fmax(xc0 - tau.x * (cj - g0), lo0), hi0);
+        const double xp1 = fmin(fmax(xc1 - tau.y * (cj - g1), lo1), hi1);
+        st2(S.xbar + e, make_double2(2.0 * xp0 - xc0, 2.0 * xp1 - xc1), st0(), st1());
         if constexpr (MAJOR) {
-            st2(S.X1 + e, make_double2(xp0, xp1), k0, k1);
-            st2(S.DX + e, make_double2(xp0 - xc0, xp1 - xc1), k0, k1);
-            st2(S.G + e, make_double2(g0, g1), k0, k1);
+            st2(S.X1 + e, make_double2(xp0, xp1), st0(), st1());
+            st2(S.DX + e, make_double2(xp0 - xc0, xp1 - xc1), st0(), st1());
+            st2(S.G + e, make_double2(g0, g1), st0(), st1());
         }
+    };
+    if (coop) {                                                // warp 0, the chunk's one row
+        trip(0, cg0, cg1, [](int, double&, double&) {});
+        return;
+    }
+    // Whether the entries sit in shared memory is the same for the whole CTA: choosing the loop here keeps the
+    // choice (and its pointer) out of the registers that are live across a trip's gathers.
+    const int ntrips = frz ? s_nrows : r1 - r0;                // frozen columns rest at their bound for the whole tile
+    if (sl.se) {
+        const int4* const E = sl.se - sl.base;
+        for (int k = warp; k < ntrips; k += kWarps)
+            trip(k, 0.0, 0.0, [&](const int lr, double& g0, double& g1) {
+                dot2_entries<true, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.y, g0, g1, kBlk, yoff);
+            });
+    } else {
+        const int4* const E = reinterpret_cast<const int4*>(cent);
+        for (int k = warp; k < ntrips; k += kWarps)
+            trip(k, 0.0, 0.0, [&](const int lr, double& g0, double& g1) {
+                dot2_entries<false, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.y, g0, g1, kBlk, yoff);
+            });
     }
 }
 
@@ -870,6 +990,9 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
     const bool k1 = node + 1 < S.B && S.fin[node + 1] == 0;
     const unsigned live = __ballot_sync(0xffffffffu, k0 || k1);
     if (live == 0) return;
+    const unsigned run0 = __ballot_sync(0xffffffffu, k0), run1 = __ballot_sync(0xffffffffu, k1);   // as in k_primal2
+    auto st0 = [&] { return ((run0 >> (threadIdx.x & 31)) & 1u) != 0; };
+    auto st1 = [&] { return ((run1 >> (threadIdx.x & 31)) & 1u) != 0; };
     double w0 = 0, w1 = 0, sig0 = 0, sig1 = 0;
     if (k0) {
         const int s = S.sbase[node] + it;
@@ -881,6 +1004,10 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
         w1 = (double)(s + 1) / (double)(s + 2);
         sig1 = S.eta[node + 1] * S.omega[node + 1];
     }
+    if (warp == 0) {                                           // every warp has the same; read back after the stage
+        s_wv[lane] = make_double2(w0, w1);
+        s_sv[lane] = make_double2(sig0, sig1);
+    }
     const int r0 = __ldg(chunk_ptr + 2 * blockIdx.x);
     const int r1 = __ldg(chunk_ptr + 2 * blockIdx.x + 1);
     const bool frz = !MAJOR && S.rfrz != nullptr;
@@ -889,11 +1016,13 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
     // into rconst once per evaluation period instead of being gathered every iteration)
     const Ent* __restrict__ aent = frz ? S.fentA + (size_t)tile * P.nnz : P.ent;
     const double* __restrict__ rconst = S.rconst + (size_t)tile * P.m;
+    const DualRowScalars rs(P, frz ? rconst : nullptr, rows_per_cta, cap);
     const Slab sl = frz ? stage_slab_frozen(P.rowptr, aent, S.fendA + (size_t)tile * P.m, S.rfrz, P.m, tile * 2, live,
-                                            r0, r1, rows_per_cta, cap)
-                        : stage_slab(P.rowptr, P.ent, r0, r1, rows_per_cta, cap);
-    const size_t base = tix(0, node, P.m);
+                                            r0, r1, rows_per_cta, cap, rs)
+                        : stage_slab(P.rowptr, P.ent, r0, r1, rows_per_cta, cap, dyn_smem, rs);
+    const unsigned base = (unsigned)tix(0, node, P.m);      // 32-bit element indices, as in k_primal2
     const double* __restrict__ xn = S.xbar + tix(0, node, P.n);
+    const unsigned xoff = (unsigned)tix(0, node, P.n);
     const bool coop = (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
     double cg0 = 0.0, cg1 = 0.0;
     if (coop) {
@@ -961,10 +1090,11 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
         return;
     }
 #endif
-    const int ntrips = frz ? s_nrows : r1 - r0;                // a frozen row's multiplier rests at zero for the whole tile
-    for (int k = warp; k < ntrips; k += kWarps) {
-        const int i = r0 + (frz ? (int)s_rows[k] : k);
-        const size_t e = base + (size_t)i * kBlk;
+    // one warp trip: row slot k of the work list; gather(k, lr, ax0, ax1) sets (ax0, ax1) to the row's A x
+    auto trip = [&](const int k, auto gather) {
+        const int lr = frz ? (int)s_rows[k] : k;
+        const int i = r0 + lr;
+        const unsigned e = base + (unsigned)i * kBlk;
         const double2 yc = ld2(S.y + e);
         const double2 a = ldcs2(S.ya + e);
         bool on0 = true, on1 = true;
@@ -973,20 +1103,39 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
             on0 = mrow[0] != 0;
             on1 = mrow[1] != 0;
         }
-        double ax0 = cg0, ax1 = cg1;
-        if (!coop) {
-            if (frz) ax0 = ax1 = __ldg(rconst + i);
-            slab_dot2(sl, aent, i - r0, xn, ax0, ax1);
-        }
-        const double bi = __ldg(P.b + i);
-        const double yp0 = on0 ? fmax(0.0, yc.x + sig0 * (bi - ax0)) : 0.0;
-        const double yp1 = on1 ? fmax(0.0, yc.y + sig1 * (bi - ax1)) : 0.0;
-        st2(S.y + e, make_double2(fma(w0, (2.0 * yp0 - yc.x) - a.x, a.x),
-                                  fma(w1, (2.0 * yp1 - yc.y) - a.y, a.y)), k0, k1);
+        double ax0, ax1;
+        gather(k, lr, ax0, ax1);
+        const double bi = DualRowScalars::View(rows_per_cta, cap).bs[k];
+        const double2 w = s_wv[lane], sig = s_sv[lane];
+        const double yp0 = on0 ? fmax(0.0, yc.x + sig.x * (bi - ax0)) : 0.0;
+        const double yp1 = on1 ? fmax(0.0, yc.y + sig.y * (bi - ax1)) : 0.0;
+        st2(S.y + e, make_double2(fma(w.x, (2.0 * yp0 - yc.x) - a.x, a.x),
+                                  fma(w.y, (2.0 * yp1 - yc.y) - a.y, a.y)), st0(), st1());
         if constexpr (MAJOR) {
-            st2(S.Y1 + e, make_double2(yp0, yp1), k0, k1);
-            st2(S.DY + e, make_double2(yp0 - yc.x, yp1 - yc.y), k0, k1);
+            st2(S.Y1 + e, make_double2(yp0, yp1), st0(), st1());
+            st2(S.DY + e, make_double2(yp0 - yc.x, yp1 - yc.y), st0(), st1());
         }
+    };
+    if (coop) {                                                // warp 0, the chunk's one row
+        trip(0, [&](int, int, double& ax0, double& ax1) { ax0 = cg0; ax1 = cg1; });
+        return;
+    }
+    // as in k_primal2: the shared / global choice of the entries is made once per CTA
+    const int ntrips = frz ? s_nrows : r1 - r0;                // a frozen row's multiplier rests at zero for the whole tile
+    if (sl.se) {
+        const int4* const E = sl.se - sl.base;
+        for (int k = warp; k < ntrips; k += kWarps)
+            trip(k, [&](const int k_, const int lr, double& ax0, double& ax1) {
+                ax0 = ax1 = DualRowScalars::View(rows_per_cta, cap).rcs[k_];   // rconst of the row, 0 without frozen coordinates
+                dot2_entries<true, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.xbar, ax0, ax1, kBlk, xoff);
+            });
+    } else {
+        const int4* const E = reinterpret_cast<const int4*>(aent);
+        for (int k = warp; k < ntrips; k += kWarps)
+            trip(k, [&](const int k_, const int lr, double& ax0, double& ax1) {
+                ax0 = ax1 = DualRowScalars::View(rows_per_cta, cap).rcs[k_];
+                dot2_entries<false, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.xbar, ax0, ax1, kBlk, xoff);
+            });
     }
 }
 
