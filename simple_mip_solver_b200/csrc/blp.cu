@@ -18,6 +18,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "blp_kernels.cuh"
@@ -175,12 +176,27 @@ int pick_nt(int B) {
     return nt;
 }
 
+// Calls f(std::integral_constant<int, NT>{}) for a nodes-per-warp width nt from pick_nt: the kernels that keep one
+// node per lane are instantiated for these six widths.
+template <class F>
+void with_nt(int nt, F&& f) {
+    switch (nt) {
+        case 1: f(std::integral_constant<int, 1>{}); break;
+        case 2: f(std::integral_constant<int, 2>{}); break;
+        case 4: f(std::integral_constant<int, 4>{}); break;
+        case 8: f(std::integral_constant<int, 8>{}); break;
+        case 16: f(std::integral_constant<int, 16>{}); break;
+        default: f(std::integral_constant<int, 32>{}); break;
+    }
+}
+
 // Step kernels: many small CTAs in tile-major order, so the CTAs resident at one moment work on
 // one or two node tiles and the gathered vector of those tiles stays in L2 (blp_kernels.cuh).
-Plan plan_rows(int rows, int B, int rows_per_warp, int max_chunks) {
+// width: nodes of the batch, nt: nodes per warp.
+Plan plan_rows(int rows, int width, int nt, int rows_per_warp, int max_chunks) {
     Plan p;
-    p.NT = pick_nt(B);
-    p.tiles = (B + p.NT - 1) / p.NT;
+    p.NT = nt;
+    p.tiles = (width + nt - 1) / nt;
     const int pass = kWarps * (32 / p.NT);
     int rpc = pass * std::max(rows_per_warp, 1);
     if (max_chunks > 0) {
@@ -470,20 +486,6 @@ size_t carve_state(const blp_handle h, int B, void* ws, DevState* S) {
     return align_up(cv.off, 256);
 }
 
-template <int NT>
-void launch_steps_nt(const DevProb& P, const DevState& S, const Plan& pc, const Plan& pr, int it,
-                     bool major, cudaStream_t st, int which) {
-    const dim3 gc(pc.chunks, pc.tiles), gr(pr.chunks, pr.tiles);
-    if (which != 1) {
-        if (major) k_primal<NT, true><<<gc, kCtaThreads, pc.smem, st>>>(P, S, it, pc.rows_per_cta, pc.cap, pc.chunk_ptr);
-        else k_primal<NT, false><<<gc, kCtaThreads, pc.smem, st>>>(P, S, it, pc.rows_per_cta, pc.cap, pc.chunk_ptr);
-    }
-    if (which != 0) {
-        if (major) k_dual<NT, true><<<gr, kCtaThreads, pr.smem, st>>>(P, S, it, pr.rows_per_cta, pr.cap, pr.chunk_ptr);
-        else k_dual<NT, false><<<gr, kCtaThreads, pr.smem, st>>>(P, S, it, pr.rows_per_cta, pr.cap, pr.chunk_ptr);
-    }
-}
-
 // which: 0 primal only, 1 dual only, 2 both. The two-nodes-per-lane kernels can be launched for a
 // sub-range of node tiles [tile0, tile0 + ntiles) (ntiles < 0: all), see ensure_graphs.
 void launch_steps(const DevProb& P, const DevState& S, const Plan& pc, const Plan& pr, int it,
@@ -501,21 +503,17 @@ void launch_steps(const DevProb& P, const DevState& S, const Plan& pc, const Pla
         }
         return;
     }
-    switch (pc.NT) {
-        case 1: launch_steps_nt<1>(P, S, pc, pr, it, major, st, which); break;
-        case 2: launch_steps_nt<2>(P, S, pc, pr, it, major, st, which); break;
-        case 4: launch_steps_nt<4>(P, S, pc, pr, it, major, st, which); break;
-        case 8: launch_steps_nt<8>(P, S, pc, pr, it, major, st, which); break;
-        case 16: launch_steps_nt<16>(P, S, pc, pr, it, major, st, which); break;
-        default: launch_steps_nt<32>(P, S, pc, pr, it, major, st, which); break;
-    }
-}
-
-template <int NT>
-void launch_eval_nt(const DevProb& P, const DevState& S, const Plan& ec, const Plan& er,
-                    cudaStream_t st) {
-    k_eval_cols<NT><<<dim3(ec.chunks, ec.tiles), kCtaThreads, 0, st>>>(P, S, ec.rows_per_cta);
-    k_eval_rows<NT><<<dim3(er.chunks, er.tiles), kCtaThreads, 0, st>>>(P, S, er.rows_per_cta);
+    with_nt(pc.NT, [&](auto nt) {
+        const dim3 gc(pc.chunks, pc.tiles), gr(pr.chunks, pr.tiles);
+        if (which != 1) {
+            if (major) k_primal<nt, true><<<gc, kCtaThreads, pc.smem, st>>>(P, S, it, pc.rows_per_cta, pc.cap, pc.chunk_ptr);
+            else k_primal<nt, false><<<gc, kCtaThreads, pc.smem, st>>>(P, S, it, pc.rows_per_cta, pc.cap, pc.chunk_ptr);
+        }
+        if (which != 0) {
+            if (major) k_dual<nt, true><<<gr, kCtaThreads, pr.smem, st>>>(P, S, it, pr.rows_per_cta, pr.cap, pr.chunk_ptr);
+            else k_dual<nt, false><<<gr, kCtaThreads, pr.smem, st>>>(P, S, it, pr.rows_per_cta, pr.cap, pr.chunk_ptr);
+        }
+    });
 }
 
 // Recompute the frozen-coordinate flags of every 32-node block (mode: see k_freeze_cols) and their count.
@@ -557,14 +555,10 @@ int launch_freeze(const DevProb& P, const DevState& S, const FreezeArgs& F, cons
 void launch_eval(const DevProb& P, const DevState& S, const Plan& ec, const Plan& er,
                  const DecideArgs& D, int K, cudaStream_t st) {
     k_tick<<<1, 1, 0, st>>>(S, K);
-    switch (ec.NT) {
-        case 1: launch_eval_nt<1>(P, S, ec, er, st); break;
-        case 2: launch_eval_nt<2>(P, S, ec, er, st); break;
-        case 4: launch_eval_nt<4>(P, S, ec, er, st); break;
-        case 8: launch_eval_nt<8>(P, S, ec, er, st); break;
-        case 16: launch_eval_nt<16>(P, S, ec, er, st); break;
-        default: launch_eval_nt<32>(P, S, ec, er, st); break;
-    }
+    with_nt(ec.NT, [&](auto nt) {
+        k_eval_cols<nt><<<dim3(ec.chunks, ec.tiles), kCtaThreads, 0, st>>>(P, S, ec.rows_per_cta);
+        k_eval_rows<nt><<<dim3(er.chunks, er.tiles), kCtaThreads, 0, st>>>(P, S, er.rows_per_cta);
+    });
     k_decide<<<(S.B + 127) / 128, 128, 0, st>>>(P, S, D);
     const int rchunks = std::min(64, std::max(1, (std::max(P.n, P.m) + 63) / 64));
     k_apply_restart<<<dim3(rchunks, (S.ld + 31) / 32), kCtaThreads, 0, st>>>(P, S);
@@ -572,42 +566,24 @@ void launch_eval(const DevProb& P, const DevState& S, const Plan& ec, const Plan
 
 void launch_check_rows(const DevProb& P, const DevState& S, const Plan& er, int only_fresh,
                        cudaStream_t st) {
-    const dim3 g(er.chunks, er.tiles);
-    switch (er.NT) {
-        case 1: k_check_rows<1><<<g, kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh); break;
-        case 2: k_check_rows<2><<<g, kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh); break;
-        case 4: k_check_rows<4><<<g, kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh); break;
-        case 8: k_check_rows<8><<<g, kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh); break;
-        case 16: k_check_rows<16><<<g, kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh); break;
-        default: k_check_rows<32><<<g, kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh); break;
-    }
+    with_nt(er.NT, [&](auto nt) {
+        k_check_rows<nt><<<dim3(er.chunks, er.tiles), kCtaThreads, 0, st>>>(P, S, er.rows_per_cta, only_fresh);
+    });
 }
 
 void launch_harvest(const DevProb& P, const DevState& S, const DevOut& O, const Plan& ec,
                     const Plan& er, bool want_frac, cudaStream_t st, int* launches) {
     const double eps = 1e-4;      // variable_epsilon of the reference (utils/tolerance.py:2)
     if (O.x || want_frac) {
-        const dim3 g(ec.chunks, ec.tiles);
-        switch (ec.NT) {
-            case 1: k_harvest_x<1><<<g, kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta); break;
-            case 2: k_harvest_x<2><<<g, kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta); break;
-            case 4: k_harvest_x<4><<<g, kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta); break;
-            case 8: k_harvest_x<8><<<g, kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta); break;
-            case 16: k_harvest_x<16><<<g, kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta); break;
-            default: k_harvest_x<32><<<g, kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta); break;
-        }
+        with_nt(ec.NT, [&](auto nt) {
+            k_harvest_x<nt><<<dim3(ec.chunks, ec.tiles), kCtaThreads, 0, st>>>(P, S, O, eps, ec.rows_per_cta);
+        });
         ++*launches;
     }
     if (O.y) {
-        const dim3 g(er.chunks, er.tiles);
-        switch (er.NT) {
-            case 1: k_harvest_y<1><<<g, kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta); break;
-            case 2: k_harvest_y<2><<<g, kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta); break;
-            case 4: k_harvest_y<4><<<g, kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta); break;
-            case 8: k_harvest_y<8><<<g, kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta); break;
-            case 16: k_harvest_y<16><<<g, kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta); break;
-            default: k_harvest_y<32><<<g, kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta); break;
-        }
+        with_nt(er.NT, [&](auto nt) {
+            k_harvest_y<nt><<<dim3(er.chunks, er.tiles), kCtaThreads, 0, st>>>(P, S, O, er.rows_per_cta);
+        });
         ++*launches;
     }
     k_harvest_nodes<<<(S.B + 127) / 128, 128, 0, st>>>(P, S, O, ec.chunks, eps, want_frac ? 1 : 0);
@@ -619,14 +595,7 @@ void launch_harvest(const DevProb& P, const DevState& S, const DevOut& O, const 
 cudaError_t launch_period_coop(blp_handle h, const DevProb& P, const DevState& S, const Plan& pc,
                                const Plan& pr, int K, cudaStream_t st) {
     const void* fn = nullptr;
-    switch (pc.NT) {
-        case 1: fn = (const void*)k_period_coop<1>; break;
-        case 2: fn = (const void*)k_period_coop<2>; break;
-        case 4: fn = (const void*)k_period_coop<4>; break;
-        case 8: fn = (const void*)k_period_coop<8>; break;
-        case 16: fn = (const void*)k_period_coop<16>; break;
-        default: fn = (const void*)k_period_coop<32>; break;
-    }
+    with_nt(pc.NT, [&](auto nt) { fn = (const void*)k_period_coop<nt>; });
     const size_t smem = pc.smem + pr.smem;        // both slabs stay resident for the whole period
     if (smem > 200 * 1024) return cudaErrorNotSupported;
     if (smem > 48 * 1024) {
@@ -871,7 +840,9 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
     int K = K0;
     const int rpw = env_int("BLP_ROWS_PER_WARP", 8);
     int NT = pick_nt(W);     // nodes per warp; re-picked when compaction narrows the batch
-    DecideArgs D{0, 0, K, o.max_iters, o.eps_rel, o.eps_infeas,
+    // evaluation / check / harvest plans: one node per lane, re-made when compaction narrows the batch
+    Plan ec = plan_rows(P.n, W, NT, 1, kEvalChunks), er = plan_rows(P.m, W, NT, 1, kEvalChunks);
+    DecideArgs D{ec.chunks, er.chunks, K, o.max_iters, o.eps_rel, o.eps_infeas,
                  env_dbl("BLP_BETA_SUFF", 0.2), env_dbl("BLP_BETA_NEC", 0.8), env_dbl("BLP_BETA_ART", 0.36),
                  env_dbl("BLP_OMEGA_THETA", 0.05), env_dbl("BLP_OMEGA_BALANCE", 0.3),
                  env_dbl("BLP_OMEGA_DEADZONE", 0.25), o.obj_cutoff};
@@ -896,11 +867,7 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
     k_init_nodes<<<(S.ld + 127) / 128, 128, 0, st>>>(P, S);
     k_init_cols<<<elementwise_grid((size_t)P.n * S.ld), kCtaThreads, 0, st>>>(P, S, lb, ub, x0, ld_in);
     k_init_rows<<<elementwise_grid((size_t)P.m * S.ld), kCtaThreads, 0, st>>>(P, S, y0, ld_in);
-    {
-        Plan er0 = plan_rows(P.m, W, 1, kEvalChunks);
-        er0.NT = NT;
-        launch_check_rows(P, S, er0, 0, st);
-    }
+    launch_check_rows(P, S, er, 0, st);
     k_build_lumask<<<elementwise_grid((size_t)P.n * (S.ld / 32) * 32), kCtaThreads, 0, st>>>(P, S);
     k_count_active<<<(W + 127) / 128, 128, 0, st>>>(S);
     launches += 6;
@@ -909,23 +876,6 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
     CK(cudaStreamSynchronize(st));
     int active = h->h_counters[0];
 
-    // plans depend on the current batch width (compaction shrinks it); NT stays fixed for the call
-    auto make_plan = [&](int rows, int width, int rows_per_warp, int max_chunks) {
-        Plan p = plan_rows(rows, width, rows_per_warp, max_chunks);
-        const int pass = kWarps * (32 / NT);
-        p.NT = NT;
-        p.tiles = (width + NT - 1) / NT;
-        int rpc = pass * std::max(rows_per_warp, 1);
-        if (max_chunks > 0) {
-            const int need = (rows + max_chunks - 1) / max_chunks;
-            rpc = std::max(rpc, ((need + pass - 1) / pass) * pass);
-        } else {
-            while (rpc > 512 && rpc > pass) rpc -= pass;
-        }
-        p.rows_per_cta = rpc;
-        p.chunks = std::max(1, (rows + rpc - 1) / rpc);
-        return p;
-    };
     // step kernels: fewer rows per warp when the batch is narrow, so that a handful of running
     // nodes still spreads over all SMs (the per-iteration latency floor of the solve's tail)
     const bool allow_v2 = env_int("BLP_V2", 1) != 0;
@@ -941,7 +891,7 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
         const bool v2 = allow_v2 && width >= kBlk && (long)std::max(P.n, P.m) * width >= (1L << 20) &&
                         (size_t)std::max(P.n, P.m) * S.ld < ((size_t)1 << 32);
         int r = v2 ? (primal ? rpw2p : rpw2) : rpw;
-        Plan p = make_plan(rows, width, r, 0);
+        Plan p = plan_rows(rows, width, NT, r, 0);
         auto shape = [&](Plan& q, int rr) {
             if (!v2) return;
             q.V = 2;                                   // a warp = one row x 64 nodes
@@ -952,7 +902,7 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
         shape(p, r);
         while (r > 1 && (long)p.chunks * p.tiles < 148L * 12) {
             r /= 2;
-            p = make_plan(rows, width, r, 0);
+            p = plan_rows(rows, width, NT, r, 0);
             shape(p, r);
         }
         return p;
@@ -972,9 +922,6 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
         return BLP_OK;
     };
     if ((rc = finish_step_plans()) != BLP_OK) return rc;
-    Plan ec = make_plan(P.n, W, 1, kEvalChunks), er = make_plan(P.m, W, 1, kEvalChunks);
-    D.chunksC = ec.chunks;
-    D.chunksR = er.chunks;
 
     if (active < W) launch_harvest(P, S, O, ec, er, want_frac, st, &launches);    // decided at set-up
 
@@ -1097,8 +1044,8 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
                     else k_eta_reset<<<(S.ld + 127) / 128, 128, 0, st>>>(P, S), ++launches;
                 }
                 coop_rejected = false;
-                ec = make_plan(P.n, S.B, 1, kEvalChunks);
-                er = make_plan(P.m, S.B, 1, kEvalChunks);
+                ec = plan_rows(P.n, S.B, NT, 1, kEvalChunks);
+                er = plan_rows(P.m, S.B, NT, 1, kEvalChunks);
                 D.chunksC = ec.chunks;
                 D.chunksR = er.chunks;
             }
@@ -1297,6 +1244,66 @@ int stage_common(blp_handle h, int B, int W, int ld, const uint8_t* row_mask, co
     return BLP_OK;
 }
 
+// blp_solve_batch on the bounds and starts staged in h->s_lb, s_ub (s_x0, s_y0 if given), results to the host
+int solve_staged(blp_handle h, int B, int ld, bool have_x0, bool have_y0, const uint8_t* row_mask,
+                 const int32_t* int_idx, int n_int, const blp_opts* opts, double* obj, double* lower_bound,
+                 int32_t* status, int32_t* iters, double* x, double* y, int32_t* frac_idx, blp_stats* stats) {
+    const uint8_t* d_mask;
+    const int32_t* d_int;
+    int rc;
+    if ((rc = stage_common(h, B, blp_slots(B, opts), ld, row_mask, int_idx, n_int, x != nullptr, y != nullptr,
+                           &d_mask, &d_int)))
+        return rc;
+    NodeOut no = node_out(h, ld);
+    rc = blp_solve_batch(h, B, h->s_lb.as<double>(), h->s_ub.as<double>(), d_mask,
+                         have_x0 ? h->s_x0.as<double>() : nullptr, have_y0 ? h->s_y0.as<double>() : nullptr,
+                         d_int, n_int, opts, h->s_ws.p, h->s_ws.cap, no.obj, no.lower, no.status,
+                         no.iters, x ? h->s_x.as<double>() : nullptr,
+                         y ? h->s_y.as<double>() : nullptr, no.frac, stats);
+    if (rc) return rc;
+    return finish_host(h, B, ld, no, x != nullptr, y != nullptr, obj, lower_bound, status, iters, x, y, frac_idx);
+}
+
+// Bound changes of B children against their parent: child k sets the bounds of variables
+// delta_var[delta_ptr[k] .. delta_ptr[k + 1]) to delta_lb / delta_ub. `who` names the entry point in the errors.
+int check_deltas(blp_handle h, int B, const int32_t* delta_ptr, const int32_t* delta_var, const double* delta_lb,
+                 const double* delta_ub, const char* who) {
+    const int nd = delta_ptr[B];
+    if (delta_ptr[0] != 0 || nd < 0 || (nd > 0 && (!delta_var || !delta_lb || !delta_ub)))
+        return fail(BLP_ERR_ARG, "%s: bad delta arrays", who);
+    for (int k = 0; k < B; ++k)
+        if (delta_ptr[k + 1] < delta_ptr[k]) return fail(BLP_ERR_ARG, "%s: delta_ptr not monotone", who);
+    for (int p = 0; p < nd; ++p)
+        if (delta_var[p] < 0 || delta_var[p] >= h->n)
+            return fail(BLP_ERR_ARG, "%s: delta_var[%d] = %d out of range", who, p, delta_var[p]);
+    return BLP_OK;
+}
+
+struct DevDeltas {
+    const int32_t* ptr;
+    const int32_t* var;
+    const double *lb, *ub;
+};
+
+// Uploads checked delta arrays with nd = delta_ptr[B] > 0 entries into h->s_delta.
+int stage_deltas(blp_handle h, int B, const int32_t* delta_ptr, const int32_t* delta_var, const double* delta_lb,
+                 const double* delta_ub, DevDeltas* out) {
+    cudaStream_t st = h->stream;
+    const int nd = delta_ptr[B];
+    const size_t ip = align_up((size_t)(B + 1) * sizeof(int32_t), 8), iv = align_up((size_t)nd * sizeof(int32_t), 8);
+    CK(h->s_delta.ensure(ip + iv + 2 * (size_t)nd * sizeof(double) + 64));
+    char* d = h->s_delta.as<char>();
+    out->ptr = reinterpret_cast<const int32_t*>(d);
+    out->var = reinterpret_cast<const int32_t*>(d + ip);
+    out->lb = reinterpret_cast<const double*>(d + ip + iv);
+    out->ub = out->lb + nd;
+    CK(cudaMemcpyAsync(d, delta_ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + ip, delta_var, nd * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + ip + iv, delta_lb, nd * sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + ip + iv + nd * sizeof(double), delta_ub, nd * sizeof(double), cudaMemcpyHostToDevice, st));
+    return BLP_OK;
+}
+
 }  // namespace
 
 int blp_solve_batch_host(blp_handle h, int B, const double* lb, const double* ub,
@@ -1313,19 +1320,8 @@ int blp_solve_batch_host(blp_handle h, int B, const double* lb, const double* ub
     if ((rc = stage_in(h, h->s_ub, ub, B, n, ld))) return rc;
     if (x0 && (rc = stage_in(h, h->s_x0, x0, B, n, ld))) return rc;
     if (y0 && (rc = stage_in(h, h->s_y0, y0, B, m, ld))) return rc;
-    const uint8_t* d_mask;
-    const int32_t* d_int;
-    if ((rc = stage_common(h, B, blp_slots(B, opts), ld, row_mask, int_idx, n_int, x != nullptr, y != nullptr,
-                           &d_mask, &d_int)))
-        return rc;
-    NodeOut no = node_out(h, ld);
-    rc = blp_solve_batch(h, B, h->s_lb.as<double>(), h->s_ub.as<double>(), d_mask,
-                         x0 ? h->s_x0.as<double>() : nullptr, y0 ? h->s_y0.as<double>() : nullptr,
-                         d_int, n_int, opts, h->s_ws.p, h->s_ws.cap, no.obj, no.lower, no.status,
-                         no.iters, x ? h->s_x.as<double>() : nullptr,
-                         y ? h->s_y.as<double>() : nullptr, no.frac, stats);
-    if (rc) return rc;
-    return finish_host(h, B, ld, no, x != nullptr, y != nullptr, obj, lower_bound, status, iters, x, y, frac_idx);
+    return solve_staged(h, B, ld, x0 != nullptr, y0 != nullptr, row_mask, int_idx, n_int, opts, obj, lower_bound,
+                        status, iters, x, y, frac_idx, stats);
 }
 
 int blp_solve_children_host(blp_handle h, int B, const double* parent_lb, const double* parent_ub,
@@ -1338,14 +1334,8 @@ int blp_solve_children_host(blp_handle h, int B, const double* parent_lb, const 
     if (!h) return fail(BLP_ERR_ARG, "blp_solve_children_host: NULL handle");
     if (B < 1 || !parent_lb || !parent_ub || !delta_ptr)
         return fail(BLP_ERR_ARG, "blp_solve_children_host: need B >= 1, parent bounds and delta_ptr");
-    const int nd = delta_ptr[B];
-    if (delta_ptr[0] != 0 || nd < 0 || (nd > 0 && (!delta_var || !delta_lb || !delta_ub)))
-        return fail(BLP_ERR_ARG, "blp_solve_children_host: bad delta arrays");
-    for (int k = 0; k < B; ++k)
-        if (delta_ptr[k + 1] < delta_ptr[k]) return fail(BLP_ERR_ARG, "blp_solve_children_host: delta_ptr not monotone");
-    for (int p = 0; p < nd; ++p)
-        if (delta_var[p] < 0 || delta_var[p] >= h->n)
-            return fail(BLP_ERR_ARG, "blp_solve_children_host: delta_var[%d] = %d out of range", p, delta_var[p]);
+    int rc = check_deltas(h, B, delta_ptr, delta_var, delta_lb, delta_ub, "blp_solve_children_host");
+    if (rc) return rc;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     const int ld = blp_ld(B), n = h->n, m = h->A0.rows;
@@ -1369,36 +1359,15 @@ int blp_solve_children_host(blp_handle h, int B, const double* parent_lb, const 
         CK(h->s_y0.ensure((size_t)m * ld * sizeof(double)));
         k_broadcast_rows<<<grow, kCtaThreads, 0, st>>>(par + 3 * n, m, ld, h->s_y0.as<double>());
     }
-    if (nd > 0) {
-        const size_t ip = align_up((size_t)(B + 1) * sizeof(int32_t), 8);
-        const size_t iv = align_up((size_t)nd * sizeof(int32_t), 8);
-        CK(h->s_delta.ensure(ip + iv + 2 * (size_t)nd * sizeof(double)));
-        char* d = h->s_delta.as<char>();
-        CK(cudaMemcpyAsync(d, delta_ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d + ip, delta_var, nd * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d + ip + iv, delta_lb, nd * sizeof(double), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d + ip + iv + nd * sizeof(double), delta_ub, nd * sizeof(double), cudaMemcpyHostToDevice, st));
-        k_patch_bounds<<<(B + 127) / 128, 128, 0, st>>>(
-            B, ld, reinterpret_cast<int32_t*>(d), reinterpret_cast<int32_t*>(d + ip),
-            reinterpret_cast<double*>(d + ip + iv),
-            reinterpret_cast<double*>(d + ip + iv + nd * sizeof(double)), h->s_lb.as<double>(),
-            h->s_ub.as<double>());
+    if (delta_ptr[B] > 0) {
+        DevDeltas d;
+        if ((rc = stage_deltas(h, B, delta_ptr, delta_var, delta_lb, delta_ub, &d))) return rc;
+        k_patch_bounds<<<(B + 127) / 128, 128, 0, st>>>(B, ld, d.ptr, d.var, d.lb, d.ub, h->s_lb.as<double>(),
+                                                         h->s_ub.as<double>());
     }
     CK(cudaGetLastError());
-    const uint8_t* d_mask;
-    const int32_t* d_int;
-    int rc;
-    if ((rc = stage_common(h, B, blp_slots(B, opts), ld, row_mask, int_idx, n_int, x != nullptr, y != nullptr,
-                           &d_mask, &d_int)))
-        return rc;
-    NodeOut no = node_out(h, ld);
-    rc = blp_solve_batch(h, B, h->s_lb.as<double>(), h->s_ub.as<double>(), d_mask,
-                         x0 ? h->s_x0.as<double>() : nullptr, y0 ? h->s_y0.as<double>() : nullptr,
-                         d_int, n_int, opts, h->s_ws.p, h->s_ws.cap, no.obj, no.lower, no.status,
-                         no.iters, x ? h->s_x.as<double>() : nullptr,
-                         y ? h->s_y.as<double>() : nullptr, no.frac, stats);
-    if (rc) return rc;
-    return finish_host(h, B, ld, no, x != nullptr, y != nullptr, obj, lower_bound, status, iters, x, y, frac_idx);
+    return solve_staged(h, B, ld, x0 != nullptr, y0 != nullptr, row_mask, int_idx, n_int, opts, obj, lower_bound,
+                        status, iters, x, y, frac_idx, stats);
 }
 
 int blp_spmv(blp_handle h, int B, int transpose, const double* X, double* Y) {
@@ -1419,17 +1388,11 @@ int blp_spmv(blp_handle h, int B, int transpose, const double* X, double* Y) {
         CK(cudaGetLastError());
         return BLP_OK;
     }
-    Plan p = plan_rows(rows, B, env_int("BLP_ROWS_PER_WARP", 8), 0);
+    Plan p = plan_rows(rows, B, pick_nt(B), env_int("BLP_ROWS_PER_WARP", 8), 0);
     plan_slab(p, transpose ? h->hptrAT : h->hptrA, rows);
-    const dim3 g(p.chunks, p.tiles);
-    switch (p.NT) {
-        case 1: k_spmv<1><<<g, kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap); break;
-        case 2: k_spmv<2><<<g, kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap); break;
-        case 4: k_spmv<4><<<g, kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap); break;
-        case 8: k_spmv<8><<<g, kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap); break;
-        case 16: k_spmv<16><<<g, kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap); break;
-        default: k_spmv<32><<<g, kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap); break;
-    }
+    with_nt(p.NT, [&](auto nt) {
+        k_spmv<nt><<<dim3(p.chunks, p.tiles), kCtaThreads, p.smem, st>>>(ptr, ent, rows, B, ld, X, Y, p.rows_per_cta, p.cap);
+    });
     CK(cudaGetLastError());
     return BLP_OK;
 }
@@ -1674,14 +1637,8 @@ int blp_simplex_children_host(blp_handle h, int B, const double* parent_lb, cons
         return fail(BLP_ERR_ARG, "blp_simplex_children_host: need parent bounds and delta_ptr");
     if ((col_status == nullptr) != (row_status == nullptr))
         return fail(BLP_ERR_ARG, "blp_simplex_children_host: col_status and row_status come together");
+    if ((rcode = check_deltas(h, B, delta_ptr, delta_var, delta_lb, delta_ub, "blp_simplex_children_host"))) return rcode;
     const int nd = delta_ptr[B];
-    if (delta_ptr[0] != 0 || nd < 0 || (nd > 0 && (!delta_var || !delta_lb || !delta_ub)))
-        return fail(BLP_ERR_ARG, "blp_simplex_children_host: bad delta arrays");
-    for (int k = 0; k < B; ++k)
-        if (delta_ptr[k + 1] < delta_ptr[k]) return fail(BLP_ERR_ARG, "blp_simplex_children_host: delta_ptr not monotone");
-    for (int p = 0; p < nd; ++p)
-        if (delta_var[p] < 0 || delta_var[p] >= h->n)
-            return fail(BLP_ERR_ARG, "blp_simplex_children_host: delta_var[%d] = %d out of range", p, delta_var[p]);
     if (max_pivots < 0) return fail(BLP_ERR_ARG, "blp_simplex_children_host: max_pivots < 0");
     const size_t n = h->n, m = h->A0.rows, mc = m - h->m_base;
     const bool use_parent = parent_slot >= 0;
@@ -1695,9 +1652,7 @@ int blp_simplex_children_host(blp_handle h, int B, const double* parent_lb, cons
     if ((rcode = sx_carve(h, B, row_mask != nullptr, col_status != nullptr, use_parent, &S))) return rcode;
     // parent vectors [lb | ub | cs | rs | mask] and deltas go up once, the per-node arrays are built on the device
     const size_t pbytes = 2 * n * sizeof(double) + n + m + mc + 64;
-    const size_t ip = align_up((size_t)(B + 1) * sizeof(int32_t), 8), iv = align_up((size_t)nd * sizeof(int32_t), 8);
     CK(h->s_par.ensure(pbytes));
-    CK(h->s_delta.ensure(ip + iv + 2 * (size_t)nd * sizeof(double) + 64));
     char* pp = h->s_par.as<char>();
     double* d_plb = reinterpret_cast<double*>(pp);
     double* d_pub = d_plb + n;
@@ -1714,15 +1669,9 @@ int blp_simplex_children_host(blp_handle h, int B, const double* parent_lb, cons
     k_sx_expand_children<<<elementwise_grid((size_t)B * n), kCtaThreads, 0, st>>>(
         B, (int)n, (int)m, d_plb, d_pub, d_pcs, d_prs, d_pmask, (int)mc, S.lb, S.ub, S.cs, S.rs, S.mask);
     if (nd > 0) {
-        char* d = h->s_delta.as<char>();
-        CK(cudaMemcpyAsync(d, delta_ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d + ip, delta_var, nd * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d + ip + iv, delta_lb, nd * sizeof(double), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d + ip + iv + nd * sizeof(double), delta_ub, nd * sizeof(double), cudaMemcpyHostToDevice, st));
-        k_sx_patch_children<<<(B + 127) / 128, 128, 0, st>>>(
-            B, (int)n, reinterpret_cast<int32_t*>(d), reinterpret_cast<int32_t*>(d + ip),
-            reinterpret_cast<double*>(d + ip + iv), reinterpret_cast<double*>(d + ip + iv + nd * sizeof(double)),
-            S.lb, S.ub);
+        DevDeltas d;
+        if ((rcode = stage_deltas(h, B, delta_ptr, delta_var, delta_lb, delta_ub, &d))) return rcode;
+        k_sx_patch_children<<<(B + 127) / 128, 128, 0, st>>>(B, (int)n, d.ptr, d.var, d.lb, d.ub, S.lb, S.ub);
     }
     if (use_parent) {
         std::vector<int32_t> par(B, parent_slot);

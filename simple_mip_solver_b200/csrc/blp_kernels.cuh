@@ -604,62 +604,6 @@ __device__ __forceinline__ void coop_dot2(const Slab& sl, const Ent* __restrict_
     }
 }
 
-// The same gather-dot for TWO rows of the slab at once: the gathers of both rows' current batches are
-// issued before either is consumed, so a warp has up to 2 * BLP_U gathers in flight. Rows of A' have
-// ~4 entries at the C5 shape — one batch — which suggested that a warp walking them one at a time has
-// too few bytes in flight (profiles/r1e: long-scoreboard stalls, no unit saturated; the round-1 review
-// asked for exactly this experiment). MEASURED (profiles/r2c_ab_pair.log, C5, 512 nodes, bit-identical
-// results): 0.560 us per node-iteration for one row per trip at 5 CTAs/SM (48 registers) against 0.601
-// (pairs, 3 CTAs/SM, 80 registers), 0.621 (pairs, 4 CTAs/SM, 64 registers), 0.650 (pairs forced to 48
-// registers, spills) and 0.652-0.673 with the dual step paired as well. More bytes in flight per warp
-// do not pay for the warps they cost; the default stays one row per trip. Kept behind BLP_PAIR_ROWS.
-// Each row's sum runs over its entries in ascending order with the same fma sequence as dot2_entries.
-template <bool SHARED>
-__device__ __forceinline__ void dot2_entries_pair(const int4* __restrict__ E, int pa, const int pa1, int pb,
-                                                  const int pb1, const double* __restrict__ Vn, double& ga0,
-                                                  double& ga1, double& gb0, double& gb1) {
-    constexpr int kU = BLP_U;
-    while (pa < pa1 || pb < pb1) {
-        double2 va[kU], vb[kU];
-#pragma unroll
-        for (int q = 0; q < kU; ++q) {
-            va[q] = make_double2(0.0, 0.0);
-            if (pa + q < pa1) {
-                const int col = SHARED ? E[pa + q].x : __ldg(&E[pa + q].x);
-                va[q] = ld2(Vn + (size_t)col * kBlk);
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < kU; ++q) {
-            vb[q] = make_double2(0.0, 0.0);
-            if (pb + q < pb1) {
-                const int col = SHARED ? E[pb + q].x : __ldg(&E[pb + q].x);
-                vb[q] = ld2(Vn + (size_t)col * kBlk);
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < kU; ++q)
-            if (pa + q < pa1) {
-                const int2 c = SHARED ? *reinterpret_cast<const int2*>(&E[pa + q].z)
-                                      : __ldg(reinterpret_cast<const int2*>(&E[pa + q].z));
-                const double cf = __hiloint2double(c.y, c.x);
-                ga0 = fma(cf, va[q].x, ga0);
-                ga1 = fma(cf, va[q].y, ga1);
-            }
-#pragma unroll
-        for (int q = 0; q < kU; ++q)
-            if (pb + q < pb1) {
-                const int2 c = SHARED ? *reinterpret_cast<const int2*>(&E[pb + q].z)
-                                      : __ldg(reinterpret_cast<const int2*>(&E[pb + q].z));
-                const double cf = __hiloint2double(c.y, c.x);
-                gb0 = fma(cf, vb[q].x, gb0);
-                gb1 = fma(cf, vb[q].y, gb1);
-            }
-        pa += kU;
-        pb += kU;
-    }
-}
-
 // Frozen coordinates of a CTA's chunk (rows [r0, r1) of the node tile whose 32-node blocks are h0, h0 + 1): one
 // byte per row in shared memory, 1 = both blocks agree (a block without a running node agrees to everything).
 // `live` is the warp's ballot of running lanes: lanes 0-15 hold the nodes of block h0, lanes 16-31 those of h0 + 1.
@@ -736,16 +680,6 @@ __device__ __forceinline__ Slab stage_slab_frozen(const int32_t* __restrict__ pt
     return s;
 }
 
-#ifndef BLP_PAIR_ROWS
-#define BLP_PAIR_ROWS 0       // 1: a warp of the primal step keeps two rows in flight (measured slower, see below)
-#endif
-#ifndef BLP_PAIR_ROWS_DUAL
-#define BLP_PAIR_ROWS_DUAL 0  // dual step: rows of A have ~10 entries (2-3 batches); pairing measured separately
-#endif
-#ifndef BLP_MINB2P
-#define BLP_MINB2P 4          // resident CTAs per SM the paired primal kernel is compiled for
-#endif
-
 // What a warp's trip over one row reads besides the row's state and gathers, staged with the slab (no round trip of
 // its own) and read from shared memory after the gathers are issued. At 48 registers (5 CTAs per SM) the compiler
 // can only keep a full BLP_U batch of gathers in flight when nothing else is live across them: with these scalars
@@ -809,7 +743,7 @@ struct DualRowScalars {
 };
 
 template <bool MAJOR>
-__global__ void __launch_bounds__(kCtaThreads, BLP_PAIR_ROWS ? BLP_MINB2P : BLP_MINB2)
+__global__ void __launch_bounds__(kCtaThreads, BLP_MINB2)
 k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_cta, const int cap,
           const int* __restrict__ chunk_ptr, const int tile0) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -852,9 +786,6 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
     const unsigned base = (unsigned)tix(0, node, P.n);
     const double* __restrict__ yn = S.y + tix(0, node, P.m);
     const unsigned yoff = (unsigned)tix(0, node, P.m);
-#if BLP_PAIR_ROWS
-    const size_t fblk = (size_t)(node >> 5) * P.n;
-#endif
     const unsigned bit = node & 31;
     const int half = lane >> 4;                                // lanes 16-31: nodes of block h0 + 1
     const bool coop = (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
@@ -864,67 +795,6 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
         coop_dot2(sl, cent, yn, warp, lane, cg0, cg1);
         if (warp != 0) return;
     }
-#if BLP_PAIR_ROWS
-    if (!coop && !frz) {
-        // two rows per trip: rows j and j + kWarps. All streaming loads and the gathers of both rows
-        // are issued before the first result is needed.
-        for (int j = r0 + warp; j < r1; j += 2 * kWarps) {
-            const int jb = j + kWarps;
-            const bool hb = jb < r1;
-            const size_t ea = base + (size_t)j * kBlk, eb = base + (size_t)(hb ? jb : j) * kBlk;
-            const double2 xba = ld2(S.xbar + ea), xbb = ld2(S.xbar + eb);
-            const double2 aa = ldcs2(S.xa + ea), ab = ldcs2(S.xa + eb);
-            const int jb_ = hb ? jb : j;
-            const uint32_t mka = (__ldg(S.lumask + fblk + j) >> bit) & 3u;
-            const uint32_t mkb = (__ldg(S.lumask + fblk + jb_) >> bit) & 3u;
-            double loa0 = __ldg(S.lref + fblk + j), hia0 = __ldg(S.uref + fblk + j);
-            double lob0 = __ldg(S.lref + fblk + jb_), hib0 = __ldg(S.uref + fblk + jb_);
-            double loa1 = loa0, hia1 = hia0, lob1 = lob0, hib1 = hib0;
-            if (mka) {
-                const double2 l2 = ldcs2(S.l + ea), u2 = ldcs2(S.u + ea);
-                if (mka & 1u) { loa0 = l2.x; hia0 = u2.x; }
-                if (mka & 2u) { loa1 = l2.y; hia1 = u2.y; }
-            }
-            if (mkb) {
-                const double2 l2 = ldcs2(S.l + eb), u2 = ldcs2(S.u + eb);
-                if (mkb & 1u) { lob0 = l2.x; hib0 = u2.x; }
-                if (mkb & 2u) { lob1 = l2.y; hib1 = u2.y; }
-            }
-            double ga0 = 0.0, ga1 = 0.0, gb0 = 0.0, gb1 = 0.0;
-            {
-                const int pa = sl.sp[j - r0], pa1 = sl.sp[j - r0 + 1];
-                const int pb = hb ? sl.sp[jb - r0] : 0, pb1 = hb ? sl.sp[jb - r0 + 1] : 0;
-                if (sl.se) dot2_entries_pair<true>(sl.se - sl.base, pa, pa1, pb, pb1, yn, ga0, ga1, gb0, gb1);
-                else dot2_entries_pair<false>(reinterpret_cast<const int4*>(P.cent), pa, pa1, pb, pb1, yn, ga0, ga1, gb0, gb1);
-            }
-            {
-                const double cj = __ldg(P.c + j);
-                const double xc0 = fma(w0, xba.x - aa.x, aa.x), xc1 = fma(w1, xba.y - aa.y, aa.y);
-                const double xp0 = fmin(fmax(xc0 - tau0 * (cj - ga0), loa0), hia0);
-                const double xp1 = fmin(fmax(xc1 - tau1 * (cj - ga1), loa1), hia1);
-                st2(S.xbar + ea, make_double2(2.0 * xp0 - xc0, 2.0 * xp1 - xc1), k0, k1);
-                if constexpr (MAJOR) {
-                    st2(S.X1 + ea, make_double2(xp0, xp1), k0, k1);
-                    st2(S.DX + ea, make_double2(xp0 - xc0, xp1 - xc1), k0, k1);
-                    st2(S.G + ea, make_double2(ga0, ga1), k0, k1);
-                }
-            }
-            if (hb) {
-                const double cj = __ldg(P.c + jb);
-                const double xc0 = fma(w0, xbb.x - ab.x, ab.x), xc1 = fma(w1, xbb.y - ab.y, ab.y);
-                const double xp0 = fmin(fmax(xc0 - tau0 * (cj - gb0), lob0), hib0);
-                const double xp1 = fmin(fmax(xc1 - tau1 * (cj - gb1), lob1), hib1);
-                st2(S.xbar + eb, make_double2(2.0 * xp0 - xc0, 2.0 * xp1 - xc1), k0, k1);
-                if constexpr (MAJOR) {
-                    st2(S.X1 + eb, make_double2(xp0, xp1), k0, k1);
-                    st2(S.DX + eb, make_double2(xp0 - xc0, xp1 - xc1), k0, k1);
-                    st2(S.G + eb, make_double2(gb0, gb1), k0, k1);
-                }
-            }
-        }
-        return;
-    }
-#endif
     // one warp trip: row slot k of the work list; gather(lr, g0, g1) adds the row's gather-dot to (g0, g1)
     auto trip = [&](const int k, double g0, double g1, auto gather) {
         const int lr = frz ? (int)s_rows[k] : k;
@@ -981,7 +851,7 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
 }
 
 template <bool MAJOR>
-__global__ void __launch_bounds__(kCtaThreads, BLP_PAIR_ROWS_DUAL ? BLP_MINB2P : BLP_MINB2)
+__global__ void __launch_bounds__(kCtaThreads, BLP_MINB2)
 k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta, const int cap,
         const int* __restrict__ chunk_ptr, const int tile0) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1035,61 +905,6 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
             cg1 += rc;
         }
     }
-#if BLP_PAIR_ROWS_DUAL
-    if (!coop && !frz) {
-        for (int i = r0 + warp; i < r1; i += 2 * kWarps) {
-            const int ib = i + kWarps;
-            const bool hb = ib < r1;
-            const int ib_ = hb ? ib : i;
-            const size_t ea = base + (size_t)i * kBlk, eb = base + (size_t)ib_ * kBlk;
-            const double2 yca = ld2(S.y + ea), ycb = ld2(S.y + eb);
-            const double2 aa = ldcs2(S.ya + ea), ab = ldcs2(S.ya + eb);
-            bool ona0 = true, ona1 = true, onb0 = true, onb1 = true;
-            if (S.rowmask) {
-                if (i >= P.m_base) {
-                    const uint8_t* mrow = S.rowmask + (size_t)(i - P.m_base) * S.ld + node;
-                    ona0 = mrow[0] != 0;
-                    ona1 = mrow[1] != 0;
-                }
-                if (ib_ >= P.m_base) {
-                    const uint8_t* mrow = S.rowmask + (size_t)(ib_ - P.m_base) * S.ld + node;
-                    onb0 = mrow[0] != 0;
-                    onb1 = mrow[1] != 0;
-                }
-            }
-            double axa0 = 0.0, axa1 = 0.0, axb0 = 0.0, axb1 = 0.0;
-            {
-                const int pa = sl.sp[i - r0], pa1 = sl.sp[i - r0 + 1];
-                const int pb = hb ? sl.sp[ib - r0] : 0, pb1 = hb ? sl.sp[ib - r0 + 1] : 0;
-                if (sl.se) dot2_entries_pair<true>(sl.se - sl.base, pa, pa1, pb, pb1, xn, axa0, axa1, axb0, axb1);
-                else dot2_entries_pair<false>(reinterpret_cast<const int4*>(P.ent), pa, pa1, pb, pb1, xn, axa0, axa1, axb0, axb1);
-            }
-            {
-                const double bi = __ldg(P.b + i);
-                const double yp0 = ona0 ? fmax(0.0, yca.x + sig0 * (bi - axa0)) : 0.0;
-                const double yp1 = ona1 ? fmax(0.0, yca.y + sig1 * (bi - axa1)) : 0.0;
-                st2(S.y + ea, make_double2(fma(w0, (2.0 * yp0 - yca.x) - aa.x, aa.x),
-                                           fma(w1, (2.0 * yp1 - yca.y) - aa.y, aa.y)), k0, k1);
-                if constexpr (MAJOR) {
-                    st2(S.Y1 + ea, make_double2(yp0, yp1), k0, k1);
-                    st2(S.DY + ea, make_double2(yp0 - yca.x, yp1 - yca.y), k0, k1);
-                }
-            }
-            if (hb) {
-                const double bi = __ldg(P.b + ib);
-                const double yp0 = onb0 ? fmax(0.0, ycb.x + sig0 * (bi - axb0)) : 0.0;
-                const double yp1 = onb1 ? fmax(0.0, ycb.y + sig1 * (bi - axb1)) : 0.0;
-                st2(S.y + eb, make_double2(fma(w0, (2.0 * yp0 - ycb.x) - ab.x, ab.x),
-                                           fma(w1, (2.0 * yp1 - ycb.y) - ab.y, ab.y)), k0, k1);
-                if constexpr (MAJOR) {
-                    st2(S.Y1 + eb, make_double2(yp0, yp1), k0, k1);
-                    st2(S.DY + eb, make_double2(yp0 - ycb.x, yp1 - ycb.y), k0, k1);
-                }
-            }
-        }
-        return;
-    }
-#endif
     // one warp trip: row slot k of the work list; gather(k, lr, ax0, ax1) sets (ax0, ax1) to the row's A x
     auto trip = [&](const int k, auto gather) {
         const int lr = frz ? (int)s_rows[k] : k;
@@ -1139,14 +954,9 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
     }
 }
 
-// Two node tiles per warp (one matrix row x 128 nodes per warp trip, the "4 nodes per lane" layout the
-// round-1 review asked for) was built and measured in commit 8a72e5b (k_primal2w / k_dual2w): results
-// bit-identical, 0.637 us per node-iteration with the primal step alone widened, 0.649 the dual step
-// alone, 0.725 both at 3-4 CTAs/SM, 0.875 at 2 CTAs/SM without spills, against 0.560 for these kernels
-// (profiles/r2e_ab_tiles2.log). Like the two-rows-per-trip variant above it halves the per-node
-// instruction count and doubles the bytes a warp has in flight, and like it it loses: what these
-// kernels need is resident WARPS, and every variant that buys per-warp parallelism with registers pays
-// in warps. Removed again; the one-row, one-tile kernels stay.
+// k_primal2 / k_dual2 walk one row x one 64-node tile per warp trip. They are bound by how many independent
+// row walks an SM holds: variants that buy per-warp parallelism with registers (two rows per trip, two node
+// tiles per warp) lose more in resident warps than they gain (DESIGN §4).
 
 // ---------------------------------------------------------------------------------------------
 // CTA-level, order-fixed reduction of per-thread accumulators into the chunk's partial slot.
