@@ -246,6 +246,25 @@ int blp_simplex_children_host(blp_handle h, int B, const double* parent_lb, cons
  * for the rows _find_gomory_cuts needs (:468-511). */
 int blp_simplex_tableau_rows_host(blp_handle h, int slot, int nrows, const int32_t* vars, double* out);
 
+/* Gomory mixed integer cuts of the previous blp_simplex_* call, one per request t: the tableau row of the
+ * basic variable vars[t] (numbered as above) in the stored factor of node slots[t] (either team: one CTA per
+ * node or a group of SMs per node), shifted / complemented to the node's final nonbasic bounds (slacks at 0),
+ * turned into a GMI cut with fractional part f0[t] in (0, 1) (col_is_int [n]: 1 for integer structurals;
+ * a shifted column stays integer only if its bound is integral), mapped back to x-space over the rows the
+ * node's LP carried (base rows and the pool rows its row mask switched on) and rounded as
+ * numerically_safe_cut(..., estimate='over'). Outputs: pi [ncuts][n], pi0 [ncuts] (the cut pi.x >= pi0) and
+ * code [ncuts]: BLP_GMI_OK, BLP_GMI_NOT_BASIC (vars[t] is not basic; pi = 0), BLP_GMI_NONFINITE (a nonbasic
+ * column sits at an infinite bound, or the cut has a non-finite coefficient or right-hand side, as a node that
+ * did not end optimal can leave behind; pi = 0) or BLP_GMI_ZERO (every coefficient is 0: pi and the unrounded
+ * pi0 are returned as numerically_safe_cut returns them). Replaces, for many nodes in one launch, the host
+ * work per cut of the reference's _find_gomory_cuts / tableau (base_node.py:468-526) and its rounding
+ * (floating_point.py:40). The arithmetic is restated in oracle/gmi_device.py, which the results match bit
+ * for bit. A slot beyond the previous call, or no stored factors on this matrix, is BLP_ERR_STATE. Slots are meant to
+ * name nodes that ended optimal (status 0); any other slot is answered too, under the rules above. */
+enum { BLP_GMI_OK = 0, BLP_GMI_NOT_BASIC = 1, BLP_GMI_NONFINITE = 2, BLP_GMI_ZERO = 3 };
+int blp_simplex_gmi_cuts_host(blp_handle h, int ncuts, const int32_t* slots, const int32_t* vars, const double* f0,
+                              const uint8_t* col_is_int, double* pi, double* pi0, int32_t* code);
+
 /* Batched SpMV on the handle's (unscaled) matrix, device pointers, node-fastest layout:
  * transpose == 0: Y[m][ld] = A X[n][ld];  transpose == 1: Y[n][ld] = A' X[m][ld].
  * Exposed for parity tests and for the SpMV roofline measurement. */

@@ -20,6 +20,7 @@ from __future__ import annotations
 
 from typing import Dict, Iterable, List, Optional, Sequence, Tuple
 
+import copy
 import types
 
 import numpy as np
@@ -150,6 +151,35 @@ class CyLPConstraint:
 
 
 # ------------------------------------------------------------------------------------------------
+class RoundMemo:
+    """Results of speculative cut rounds (``BranchAndBound(frontier_cut_rounds=True)``) for the real nodes to find.
+
+    ``lps``: (LP state key, digest of the starting basis) -> what a simplex solve of that LP from that basis
+    returns (status, objective, x, y, reduced costs, basis, pivots): a node LP's simplex solve depends on nothing
+    else. ``cuts``: (solve key, node idx, cut round, max_gomory_cuts) -> the device GMI cuts of that solve, as
+    ``BaseNode._device_gomory_cuts`` makes them while the solve's factor is in the store. A frontier prefetch
+    empties it once it holds more than ``BranchAndBound.MEMO_LPS`` LP results."""
+
+    def __init__(self):
+        self.lps: Dict[tuple, tuple] = {}
+        self.cuts: Dict[tuple, dict] = {}
+        self.lp_hits = 0
+        self.cut_hits = 0
+        self.speculative_lps = 0
+        self.cut_round_resolves = 0     # real nodes that re-solved an LP to get its factor back for cuts
+
+    def clear(self):
+        self.lps.clear()
+        self.cuts.clear()
+
+
+def _start_digest(start) -> tuple:
+    if start is None:
+        return ()
+    return (np.asarray(start[0]).tobytes(), np.asarray(start[1]).tobytes(), tuple(start[2].items()))
+
+
+# ------------------------------------------------------------------------------------------------
 class SharedLP:
     """What all node LPs of one MILP have in common: ``min c.x, A x >= b`` plus a pool of cut rows.
 
@@ -189,6 +219,7 @@ class SharedLP:
         self.root_bounds = None
         self.root_xy = None
         self.max_abs_coef = None        # max |A_ij| (BaseNode.max_term), computed on first use
+        self.memo: Optional[RoundMemo] = None   # speculative cut rounds of a frontier (BranchAndBound)
 
     @property
     def engine(self):
@@ -316,6 +347,7 @@ class CyClpSimplex:
         self._parent_ref = None         # the parent's _factor_ref (copy_for_child)
         self._parent_bounds = (None, None)   # the parent's bound arrays (children of one parent share them)
         self._basis_start = None        # setBasisStatus by row NAME: (cols, base rows, {cut name: status})
+        self._solve_start = None        # the starting basis of the last simplex solve (its RoundMemo key part)
         self.integer_indices_hint: Optional[Sequence[int]] = None
         self.integer_index_set = None           # frozenset of the hint once a node has checked it
         self.solver_opts: Dict[str, float] = {}
@@ -676,6 +708,74 @@ class CyClpSimplex:
         structurals, then the slack of every row in this LP's order), computed on the device from the
         factorised basis of the last simplex solve; None when that factor is gone (another batch was
         solved since) or the LP was not solved by the simplex path."""
+        found = self._stored_factor()
+        if found is None:
+            return None
+        slot, to_pool = found
+        rows = self._shared.engine.simplex_tableau_rows(slot, to_pool[np.asarray(variables, dtype=int)])
+        return rows[:, to_pool]
+
+    def gmi_cuts(self, variables, f0, col_is_int) -> Optional[Tuple[np.ndarray, np.ndarray, np.ndarray]]:
+        """Rounded GMI cuts of the basic ``variables`` (LP numbering, as ``tableau_rows``) with fractional
+        parts ``f0``, computed on the device from the factorised basis of the last simplex solve in one call
+        (engine.simplex_gmi_cuts): (pi [k, n], pi0 [k], code [k]), or None when that factor is gone."""
+        found = self._stored_factor()
+        if found is None:
+            return None
+        slot, to_pool = found
+        v = to_pool[np.asarray(variables, dtype=int)]
+        return self._shared.engine.simplex_gmi_cuts(np.full(len(v), slot), v, f0, col_is_int)
+
+    @property
+    def has_stored_factor(self) -> bool:
+        """True while the engine's factor store holds the factorised basis of this LP's last simplex solve."""
+        return self._stored_factor() is not None
+
+    def clone(self) -> 'CyClpSimplex':
+        """An independent copy of this LP with its last solve (a speculative cut round works on it)."""
+        c = copy.copy(self)
+        c._l, c._u = self._l.copy(), self._u.copy()
+        c._cuts, c._cut_keys = dict(self._cuts), dict(self._cut_keys)
+        c._foreign_rows, c._vars = dict(self._foreign_rows), list(self._vars)
+        return c
+
+    @property
+    def solve_key(self):
+        """RoundMemo key of the current solve: None unless the LP is solved as it stands by the simplex path."""
+        if self._solve_start is None or not self.has_exact_basis or self._solved_key != self._state_key():
+            return None
+        return self._solved_key, _start_digest(self._solve_start)
+
+    def memo_cuts(self, idx, cut_round, max_gomory_cuts):
+        """Device GMI cuts a speculative round made of this very solve, or None."""
+        sh = self._shared
+        key = self.solve_key
+        if sh is None or sh.memo is None or key is None:
+            return None
+        got = sh.memo.cuts.get((key, idx, cut_round, max_gomory_cuts))
+        if got is None:
+            return None
+        sh.memo.cut_hits += 1
+        return {r: (CyLPArray(pi), pi0) for r, (pi, pi0) in got.items()}
+
+    def restore_factor(self) -> bool:
+        """Put this LP's factor back in the store by solving it again from the basis its last solve started from
+        (the same solve, so the same result). Only while speculative cut rounds are on: a solve answered by the
+        RoundMemo, or one of an earlier chunk of a batch, left no factor where the one-node-per-call run has one."""
+        sh = self._shared
+        if sh is None or sh.memo is None or self.solve_key is None or hasattr(sh.engine, 'parts'):
+            return False
+        start = self._basis_start
+        self._basis_out, self._basis_start = None, self._solve_start
+        try:
+            solve_lps([self], force=True)
+        finally:
+            self._basis_start = start
+        return self.has_stored_factor
+
+    def _stored_factor(self):
+        """(slot of this LP in the engine's factor store, map from LP numbering to the device's pool numbering)
+        while the store still holds the factor of this LP's last solve, else None."""
         sh = self._need_shared()
         ref = self._factor_ref
         if ref is None or self._solved_key != self._state_key() or ref[0] != sh.simplex_calls \
@@ -683,9 +783,7 @@ class CyClpSimplex:
             return None
         n, m = sh.n, sh.m
         pool = [m + sh.pool_row(self, nm) for nm in self._cuts]      # pool row of every cut row of this LP
-        to_pool = np.concatenate([np.arange(n + m), n + np.asarray(pool, dtype=int)]).astype(int)
-        rows = sh.engine.simplex_tableau_rows(ref[1], to_pool[np.asarray(variables, dtype=int)])
-        return rows[:, to_pool]
+        return ref[1], np.concatenate([np.arange(n + m), n + np.asarray(pool, dtype=int)]).astype(int)
 
     def set_warm_start(self, x, duals_by_row: Dict[str, float], y_base):
         """Parent's primal vector and row duals; the analogue of handing the parent's basis to
@@ -744,6 +842,8 @@ def solve_lps(lps: Iterable[CyClpSimplex], force: bool = False) -> int:
         assert lp.solvable, 'the device solves A x >= b over one variable vector: this model has rows with an ' \
                             'upper bound, further variables or no base rows (BaseAlgorithm converts "<=" models)'
         if force or lp._solved_key is None or lp._solved_key != lp._state_key():
+            if not force and sh.memo is not None and _from_memo(sh, lp):
+                continue
             groups.setdefault(id(sh), []).append(lp)
     sent = 0
     for todo in groups.values():
@@ -756,6 +856,36 @@ def solve_lps(lps: Iterable[CyClpSimplex], force: bool = False) -> int:
             _solve_group(sh, batch, budget, default_opts)
             sent += len(batch)
     return sent
+
+
+def _memo_start(lp: CyClpSimplex):
+    """The basis a simplex solve of ``lp`` starts from (what _solve_group_simplex's start_of picks), or None when
+    the solve also depends on something else (a stored parent factor, a first-order crossover start)."""
+    if lp.solver_opts.get('factor_cache', False):
+        return None
+    return lp._basis_out if lp._basis_out is not None else lp._basis_start
+
+
+def _from_memo(sh: SharedLP, lp: CyClpSimplex) -> bool:
+    start = _memo_start(lp)
+    if start is None:
+        return False
+    got = sh.memo.lps.get((lp._state_key(), _start_digest(start)))
+    if got is None:
+        return False
+    sh.memo.lp_hits += 1
+    status, obj, x, y, rc, basis, pivots = got
+    lp._status, lp.iteration = status, pivots
+    lp._basis_out = basis
+    lp._basis_exact, lp._basis_kept, lp._factor_ref = True, None, None
+    lp._solve_start = start
+    if status == 1:
+        lp._obj, lp._x, lp._y, lp._rc, lp._lower_bound = float('inf'), None, None, None, float('inf')
+    else:
+        lp._x, lp._y, lp._rc = CyLPArray(x), y.copy(), CyLPArray(rc)
+        lp._obj = lp._lower_bound = obj
+    lp._solved_key = lp._state_key()
+    return True
 
 
 def _solve_group(sh: SharedLP, batch: List[CyClpSimplex], budget: int, default_opts):
@@ -884,10 +1014,12 @@ def _solve_group_simplex(sh: SharedLP, batch: List[CyClpSimplex], budget: int, d
     sh.lps_solved += B
     sh.kernel_launches += int(res.stats.get('kernel_launches', 1))
     sh.simplex_pivots += int(res.pivots.sum())
+    starts = [start_of(lp) for lp in batch]
     for k, lp in enumerate(batch):
         st = int(res.status[k])
         lp._status = st
         lp.iteration = int(res.pivots[k])
+        lp._solve_start = None if use_cache else starts[k]
         rows = [m + sh.pool_row(lp, nm) for nm in lp._cuts]
         lp._basis_out = (res.col_status[k].copy(), res.row_status[k, :m].copy(),
                          {nm: int(res.row_status[k, r]) for nm, r in zip(lp._cuts, rows)})
@@ -902,6 +1034,13 @@ def _solve_group_simplex(sh: SharedLP, batch: List[CyClpSimplex], budget: int, d
         lp._rc = CyLPArray(res.reduced_costs[k])
         lp._obj = float(res.objective[k])
         lp._lower_bound = lp._obj          # a dual feasible basis: c.x of the basic solution is the dual objective
+    if sh.memo is not None:
+        for lp in batch:
+            if lp._solve_start is not None:
+                key = (lp._state_key(), _start_digest(lp._solve_start))
+                sh.memo.lps[key] = (lp._status, lp._obj, None if lp._x is None else np.asarray(lp._x).copy(),
+                                    None if lp._y is None else lp._y.copy(),
+                                    None if lp._rc is None else np.asarray(lp._rc).copy(), lp._basis_out, lp.iteration)
 
 
 def _deltas_against(lp: CyClpSimplex, l0, u0, limit: int):

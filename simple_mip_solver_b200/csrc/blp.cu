@@ -236,6 +236,9 @@ struct blp_handle_s {
     DevBuf uc, ub;                     // unscaled objective / row lower bounds (simplex path)
     // dual simplex path (blp_simplex_*): factor stores of the current and the previous call, staging
     DevBuf sx_binv[2], sx_head[2], sx_stat[2], sx_wts[2], sx_work, sx_in, sx_out, sx_wide;
+    DevBuf sx_bnd[2];                  // each store's node bounds [B][n] x 2 and row masks [B][m - m_base]
+    int sx_bnd_mask[2] = {0, 0};       // ... whether that call had row masks (else every pool row was on)
+    DevBuf sx_gmi;                     // blp_simplex_gmi_cuts_host: requests and results
     int sx_cur = 0;                    // store the NEXT call writes; the other one holds the last call
     int sx_last_B = 0, sx_last_m = -1; // nodes / rows of the last call's store (-1: none)
     DevBuf chunkC, chunkR;             // row ranges of the step-kernel CTAs (primal / dual)
@@ -1511,6 +1514,18 @@ int sx_run(blp_handle h, int B, const SxStage& S, bool use_parent, int max_pivot
     Q.pBinv = h->sx_binv[prev].as<double>(); Q.phead = h->sx_head[prev].as<int32_t>();
     Q.pstat = h->sx_stat[prev].as<int8_t>(); Q.pwts = h->sx_wts[prev].as<double>();
     Q.work = h->sx_work.as<double>(); Q.work_stride = stride;
+    // The bounds and row masks stay with the store: blp_simplex_gmi_cuts_host reads a node's final bounds there.
+    // Copied on every call, asked for or not: 2 B n doubles plus B (m - m_base) bytes, device to device, against
+    // the B m^2 doubles of inverses the same call writes (at m = n = 500: 8 KB per node against 2 MB).
+    const size_t mc = (size_t)(m - h->m_base);
+    CK(h->sx_bnd[cur].ensure((size_t)2 * B * n * sizeof(double) + (size_t)B * mc));
+    {
+        double* bl = h->sx_bnd[cur].as<double>();
+        CK(cudaMemcpyAsync(bl, S.lb, (size_t)B * n * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(bl + (size_t)B * n, S.ub, (size_t)B * n * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        if (S.mask) CK(cudaMemcpyAsync(bl + (size_t)2 * B * n, S.mask, (size_t)B * mc, cudaMemcpyDeviceToDevice, st));
+        h->sx_bnd_mask[cur] = S.mask != nullptr;
+    }
     Q.obj = S.obj; Q.status = S.status; Q.pivots = S.pivots; Q.flips = S.flips;
     Q.x = S.x; Q.y = S.y; Q.rc = S.rc; Q.cstat_out = S.cso; Q.rstat_out = S.rso;
     CK(cudaEventRecord(h->ev[2], st));
@@ -1711,6 +1726,57 @@ int blp_simplex_tableau_rows_host(blp_handle h, int slot, int nrows, const int32
     return BLP_OK;
 }
 
+int blp_simplex_gmi_cuts_host(blp_handle h, int ncuts, const int32_t* slots, const int32_t* vars, const double* f0,
+                              const uint8_t* col_is_int, double* pi, double* pi0, int32_t* code) {
+    if (!h) return fail(BLP_ERR_ARG, "blp_simplex_gmi_cuts_host: NULL handle");
+    if (ncuts < 1 || !slots || !vars || !f0 || !col_is_int || !pi || !pi0 || !code)
+        return fail(BLP_ERR_ARG, "blp_simplex_gmi_cuts_host: need ncuts >= 1 and every array");
+    const int n = h->n, m = h->A0.rows, N = n + m;
+    if (h->sx_last_m != m)
+        return fail(BLP_ERR_STATE, "blp_simplex_gmi_cuts_host: no simplex call on this matrix has its factors stored");
+    for (int t = 0; t < ncuts; ++t) {
+        if (slots[t] < 0 || slots[t] >= h->sx_last_B)
+            return fail(BLP_ERR_STATE, "blp_simplex_gmi_cuts_host: slots[%d] = %d does not name a node of the previous "
+                                       "simplex call", t, slots[t]);
+        if (vars[t] < 0 || vars[t] >= N) return fail(BLP_ERR_ARG, "blp_simplex_gmi_cuts_host: vars[%d] out of range", t);
+        if (!(f0[t] > 0.0 && f0[t] < 1.0)) return fail(BLP_ERR_ARG, "blp_simplex_gmi_cuts_host: f0[%d] not in (0, 1)", t);
+    }
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    const int ldm = (m + 31) / 32 * 32;
+    const int last = h->sx_cur ^ 1;
+    const size_t B = (size_t)h->sx_last_B;
+    CK(h->sx_gmi.ensure((size_t)ncuts * (2 * sizeof(int32_t) + sizeof(double)) + (size_t)n + (size_t)ncuts * (n + 1) * sizeof(double) +
+                        (size_t)ncuts * sizeof(int32_t) + 256 * 8));
+    Carve cv{h->sx_gmi.as<char>()};
+    int32_t* d_slot = cv.take<int32_t>(ncuts);
+    int32_t* d_var = cv.take<int32_t>(ncuts);
+    double* d_f0 = cv.take<double>(ncuts);
+    uint8_t* d_int = cv.take<uint8_t>(n);
+    double* d_pi = cv.take<double>((size_t)ncuts * n);
+    double* d_pi0 = cv.take<double>(ncuts);
+    int32_t* d_code = cv.take<int32_t>(ncuts);
+    CK(cudaMemcpyAsync(d_slot, slots, ncuts * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_var, vars, ncuts * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_f0, f0, ncuts * sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_int, col_is_int, n, cudaMemcpyHostToDevice, st));
+    SxProb P{m, h->m_base, n, ldm, h->P.rowptr, h->uent.as<Ent>(), h->P.cptr, h->ucent.as<Ent>(),
+             h->uc.as<double>(), h->ub.as<double>()};
+    const double* bnd = h->sx_bnd[last].as<double>();
+    GmiArgs G{ncuts, h->sx_binv[last].as<double>(), h->sx_head[last].as<int32_t>(), h->sx_stat[last].as<int8_t>(),
+              bnd, bnd + B * n, h->sx_bnd_mask[last] ? reinterpret_cast<const uint8_t*>(bnd + 2 * B * n) : nullptr,
+              d_slot, d_var, d_f0, d_int, d_pi, d_pi0, d_code};
+    const size_t smem = (size_t)2 * m * sizeof(double);
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_simplex_gmi_cuts, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_simplex_gmi_cuts<<<ncuts, kGmiThreads, smem, st>>>(P, G);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(pi, d_pi, (size_t)ncuts * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(pi0, d_pi0, ncuts * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(code, d_code, ncuts * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return BLP_OK;
+}
+
 int blp_stream_sync(blp_handle h) {
     if (!h) return fail(BLP_ERR_ARG, "blp_stream_sync: NULL handle");
     CK(cudaSetDevice(h->device));
@@ -1794,7 +1860,8 @@ int blp_destroy(blp_handle h) {
                       &h->s_ub, &h->s_x0, &h->s_y0, &h->s_mask, &h->s_x, &h->s_y, &h->s_tmp,
                       &h->s_ws, &h->s_node, &h->s_int, &h->s_delta, &h->s_par, &h->uc, &h->ub,
                       &h->sx_binv[0], &h->sx_binv[1], &h->sx_head[0], &h->sx_head[1], &h->sx_stat[0],
-                      &h->sx_stat[1], &h->sx_wts[0], &h->sx_wts[1], &h->sx_work, &h->sx_in, &h->sx_out, &h->sx_wide};
+                      &h->sx_stat[1], &h->sx_wts[0], &h->sx_wts[1], &h->sx_work, &h->sx_in, &h->sx_out, &h->sx_wide,
+                      &h->sx_bnd[0], &h->sx_bnd[1], &h->sx_gmi};
     for (DevBuf* b : bufs) b->release();
     for (cudaEvent_t e : h->ev) if (e) cudaEventDestroy(e);
     for (cudaEvent_t e : h->ev_join) if (e) cudaEventDestroy(e);

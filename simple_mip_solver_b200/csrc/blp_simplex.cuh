@@ -908,4 +908,218 @@ __global__ void k_simplex_tableau_rows(const SxProb P, const double* __restrict_
     }
 }
 
+// ---- GMI cuts of stored factors (BaseNode._gomory_cuts_of_basis + numerically_safe_cut, on the device) ----
+constexpr int kGmiThreads = 256;           // also the lane count of the two ordered dot products
+constexpr int GMI_OK = 0, GMI_NOT_BASIC = 1, GMI_NONFINITE = 2, GMI_ZERO = 3;
+constexpr double kGmiMaxTerm = 1e3;        // utils/tolerance.py max_term
+constexpr double kGmiGoodEps = 1e-2;       // good_coefficient_approximation_epsilon
+constexpr double kGmiExactEps = 1e-14;     // exact_coefficient_approximation_epsilon
+
+// utils/floating_point.get_fraction(x, estimate): est = +1 'over', -1 'under', 0 nearest. The convergents
+// h / k are kept in doubles: a returned one has |h|, k <= max_term (|x| + 1) and is exact, and the partial
+// sums never cancel (h_i, h_{i-1}, h_{i-2} share a sign from i = 1 on, k_i > 0), so the comparison with
+// max_term decides as on Python's integers; a convergent beyond it (even an infinite one) is only compared.
+__device__ __forceinline__ void gmi_fraction(const double x, const int est, double& num, double& den) {
+    if (fabs(x) > kGmiMaxTerm) {
+        num = est > 0 ? ceil(x) : (est < 0 ? floor(x) : rint(x));
+        den = 1.0;
+        return;
+    }
+    double h2 = 0.0, k2 = 1.0, h1 = 1.0, k1 = 0.0, h, k;
+    double value = x;
+    int last = 0;
+    for (;; ++last) {
+        const double a = floor(value);
+        h = sx_add(sx_mul(a, h1), h2);
+        k = sx_add(sx_mul(a, k1), k2);
+        if (h > kGmiMaxTerm || k > kGmiMaxTerm) break;
+        const double rest = sx_sub(value, a);
+        if (rest == 0.0) { num = h; den = k; return; }        // exact
+        value = __ddiv_rn(1.0, rest);
+        h2 = h1; k2 = k1; h1 = h; k1 = k;
+    }
+    // h1 / k1 is convergent last - 1, h2 / k2 convergent last - 2 (last >= 1 here); odd ones lie above x
+    const bool odd = last & 1;
+    if (est > 0) {
+        if (!odd) { num = h1; den = k1; }
+        else if (last >= 2) { num = h2; den = k2; }
+        else { num = ceil(x); den = 1.0; }
+    } else if (est < 0) {
+        if (odd) { num = h1; den = k1; }
+        else { num = h2; den = k2; }
+    } else {
+        num = h1; den = k1;
+    }
+}
+
+// numerically_safe_cut's rounding of one scaled coefficient (estimate 'over')
+__device__ __forceinline__ double gmi_safe_coef(const double coef) {
+    double n, d;
+    gmi_fraction(coef, 1, n, d);
+    if (coef != 0.0 && fabs(sx_sub(1.0, __ddiv_rn(__ddiv_rn(n, d), coef))) > kGmiGoodEps) {
+        double n2, d2;
+        gmi_fraction(coef, 0, n2, d2);
+        if (fabs(sx_sub(__ddiv_rn(n2, d2), coef)) < kGmiExactEps) { n = n2; d = d2; }
+    }
+    return __ddiv_rn(n, d);
+}
+
+struct GmiArgs {
+    int ncuts;
+    const double* Binv; const int32_t* head; const int8_t* stat;   // the last call's store
+    const double* lb; const double* ub; const uint8_t* rowon;       // its bounds / row masks (rowon may be null)
+    const int32_t* slot; const int32_t* var; const double* f0; const uint8_t* col_is_int;
+    double* pi; double* pi0; int32_t* code;                          // [ncuts][n], [ncuts], [ncuts]
+};
+
+// One CTA (kGmiThreads threads) per request t: the GMI cut of the tableau row of basic variable var[t] of node
+// slot[t], mapped to x-space and rounded as numerically_safe_cut(estimate='over'). Restated in numpy by
+// oracle/gmi_device.py, which the results match bit for bit. Order of the floating-point work:
+//   tableau row   as k_simplex_tableau_rows: structural j = sum over the entries of column j ascending by row
+//                 of Binv(r, i) a_ij (terms with Binv(r, i) = 0 skipped), slack n + i = -Binv(r, i)
+//   GMI           row_j = tab_j sign_j (sign -1 at an upper bound), f = row - floor(row), integer:
+//                 f <= f0 ? f / f0 : (1 - f) / (1 - f0), else row > 0 ? row / f0 : -row / (1 - f0); basic -> 0;
+//                 a column is integer if col_is_int and its offset is within 1e-9 of an integer
+//   x-space       pi_j = pi'_j sign_j + sum over the entries of column j ascending by row of pi_s(i) a_ij
+//                 (pi_s(i) = 0 skipped; rows masked off for the node carry pi_s = 0)
+//   right side    (1 + sum_j pi_x(j) offset_j) + sum_i pi_s(i) b_i, each sum in 256 lanes: lane t adds the
+//                 terms t, t + 256, t + 512, ... in order, then the 256 lane sums are added in lane order
+//   rounding      scale by 1 / max|pi|, coefficients rounded over, the right side under (gmi_fraction)
+// Shared memory: row r of Binv and pi_s, 2 m doubles (dynamic, up to 128 KB at m = 8192).
+__global__ void __launch_bounds__(kGmiThreads)
+k_simplex_gmi_cuts(const SxProb P, const GmiArgs G) {
+    extern __shared__ double gmi_smem[];
+    double* rowr = gmi_smem;                 // [m]
+    double* pis = gmi_smem + P.m;            // [m]
+    __shared__ double part[kGmiThreads];
+    __shared__ int s_pos, s_bad;
+    __shared__ double s_max;
+    const int t = blockIdx.x, tid = threadIdx.x;
+    const int m = P.m, n = P.n, N = n + m, mc = m - P.m_base;
+    const int slot = G.slot[t], v = G.var[t];
+    const double f0 = G.f0[t];
+    const int8_t* st = G.stat + (size_t)slot * N;
+    const int32_t* hd = G.head + (size_t)slot * m;
+    const double* lb = G.lb + (size_t)slot * n;
+    const double* ub = G.ub + (size_t)slot * n;
+    const uint8_t* on = G.rowon ? G.rowon + (size_t)slot * mc : nullptr;
+    double* pi = G.pi + (size_t)t * n;
+    if (tid == 0) { s_pos = -1; s_bad = 0; }
+    __syncthreads();
+    for (int i = tid; i < m; i += kGmiThreads)
+        if (hd[i] == v) s_pos = i;
+    // nonbasic structurals sit at a bound (|bound| >= 1e30 is none), slacks at 0
+    for (int j = tid; j < n; j += kGmiThreads) {
+        if (st[j] == SX_BASIC) continue;
+        const double o = st[j] == SX_UPPER ? ub[j] : lb[j];
+        if (!isfinite(o) || fabs(o) >= 1e30) s_bad = 1;
+    }
+    __syncthreads();
+    const int r = s_pos;
+    if (r < 0 || s_bad) {
+        for (int j = tid; j < n; j += kGmiThreads) pi[j] = 0.0;
+        if (tid == 0) { G.pi0[t] = 0.0; G.code[t] = r < 0 ? GMI_NOT_BASIC : GMI_NONFINITE; }
+        return;
+    }
+    const double* Br = G.Binv + (size_t)slot * m * P.ldm + (size_t)r * P.ldm;
+    for (int i = tid; i < m; i += kGmiThreads) rowr[i] = Br[i];
+    __syncthreads();
+    const double omf0 = sx_sub(1.0, f0);
+    // slacks: offset 0, sign +1, never integer
+    double acc_b = 0.0;
+    for (int i = tid; i < m; i += kGmiThreads) {
+        double ps = 0.0;
+        const bool carried = !(i >= P.m_base && on && on[i - P.m_base] == 0);
+        if (st[n + i] != SX_BASIC) {
+            const double row = sx_mul(-rowr[i], 1.0);
+            ps = row > 0.0 ? __ddiv_rn(row, f0) : __ddiv_rn(-row, omf0);
+        }
+        if (!carried) ps = 0.0;
+        pis[i] = ps;
+        acc_b = sx_add(acc_b, sx_mul(ps, P.b[i]));
+    }
+    __syncthreads();
+    // structurals
+    double acc_o = 0.0, big = 0.0;
+    for (int j = tid; j < n; j += kGmiThreads) {
+        const int8_t s = st[j];
+        const int p0 = P.cptr[j], p1 = P.cptr[j + 1];
+        double px = 0.0, off = 0.0, sign = 1.0;
+        if (s != SX_BASIC) {
+            sign = s == SX_UPPER ? -1.0 : 1.0;
+            off = s == SX_UPPER ? ub[j] : lb[j];
+            double tab = 0.0;
+            for (int p = p0; p < p1; ++p) {
+                const Ent e = P.cent[p];
+                const double ri = rowr[e.idx];
+                if (ri != 0.0) tab = sx_add(tab, sx_mul(ri, e.val));
+            }
+            const double row = sx_mul(tab, sign);
+            const bool is_int = G.col_is_int[j] && fabs(sx_sub(off, rint(off))) <= 1e-9;
+            double ps;
+            if (is_int) {
+                const double f = sx_sub(row, floor(row));
+                ps = f <= f0 ? __ddiv_rn(f, f0) : __ddiv_rn(sx_sub(1.0, f), omf0);
+            } else {
+                ps = row > 0.0 ? __ddiv_rn(row, f0) : __ddiv_rn(-row, omf0);
+            }
+            px = sx_mul(ps, sign);
+        }
+        acc_o = sx_add(acc_o, sx_mul(px, off));
+        double as = 0.0;
+        for (int p = p0; p < p1; ++p) {
+            const Ent e = P.cent[p];
+            const double ps = pis[e.idx];
+            if (ps != 0.0) as = sx_add(as, sx_mul(ps, e.val));
+        }
+        const double coef = sx_add(px, as);
+        pi[j] = coef;
+        if (!isfinite(coef)) s_bad = 1;
+        big = fmax(big, fabs(coef));
+    }
+    // right-hand side: lane sums in lane order
+    part[tid] = acc_o;
+    __syncthreads();
+    double dot_o = 0.0;
+    if (tid == 0)
+        for (int l = 0; l < kGmiThreads; ++l) dot_o = sx_add(dot_o, part[l]);
+    __syncthreads();
+    part[tid] = acc_b;
+    __syncthreads();
+    if (tid == 0) {
+        double dot_b = 0.0;
+        for (int l = 0; l < kGmiThreads; ++l) dot_b = sx_add(dot_b, part[l]);
+        part[0] = sx_add(sx_add(1.0, dot_o), dot_b);
+    }
+    __syncthreads();
+    const double rhs = part[0];
+    // a non-finite coefficient or right-hand side (a factor that is not a clean solve's) gives no cut: the
+    // rounding below is only defined on finite values
+    if (s_bad || !isfinite(rhs)) {
+        for (int j = tid; j < n; j += kGmiThreads) pi[j] = 0.0;
+        if (tid == 0) { G.pi0[t] = 0.0; G.code[t] = GMI_NONFINITE; }
+        return;
+    }
+    // largest |coefficient| (order independent)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) big = fmax(big, __shfl_xor_sync(0xffffffffu, big, o));
+    if (tid == 0) s_max = 0.0;
+    __syncthreads();
+    if ((tid & 31) == 0) atomicMax(reinterpret_cast<unsigned long long*>(&s_max), __double_as_longlong(big));
+    __syncthreads();
+    const double biggest = s_max;            // >= 0, so the bit patterns order as the values
+    if (biggest == 0.0) {                    // numerically_safe_cut returns a zero cut unchanged
+        if (tid == 0) { G.pi0[t] = rhs; G.code[t] = GMI_ZERO; }
+        return;
+    }
+    const double factor = __ddiv_rn(1.0, biggest);
+    for (int j = tid; j < n; j += kGmiThreads) pi[j] = gmi_safe_coef(sx_mul(pi[j], factor));
+    if (tid == 0) {
+        double nu, de;
+        gmi_fraction(sx_mul(rhs, factor), -1, nu, de);
+        G.pi0[t] = __ddiv_rn(nu, de);
+        G.code[t] = GMI_OK;
+    }
+}
+
 }  // namespace blp

@@ -25,6 +25,9 @@ _lib = None
 
 INF = 1e30   # |bound| >= INF means "no bound" on the device side
 
+# codes of BatchLP.simplex_gmi_cuts (BLP_GMI_* of include/blp.h)
+GMI_OK, GMI_NOT_BASIC, GMI_NONFINITE, GMI_ZERO = 0, 1, 2, 3
+
 
 class BlpError(RuntimeError):
     pass
@@ -75,6 +78,7 @@ _SIGNATURES = {
     'blp_simplex_children_host': (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int,
                                             _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(BlpStats)]),
     'blp_simplex_tableau_rows_host': (C.c_int, [_P, C.c_int, C.c_int, _P, _P]),
+    'blp_simplex_gmi_cuts_host': (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P, _P, _P]),
     'blp_spmv': (C.c_int, [_P, C.c_int, C.c_int, _P, _P]),
     'blp_stream': (_P, [_P]),
     'blp_stream_sync': (C.c_int, [_P]),
@@ -421,6 +425,24 @@ class BatchLP:
                'blp_simplex_tableau_rows_host')
         return out
 
+    def simplex_gmi_cuts(self, slots, variables, f0, int_mask):
+        """Rounded GMI cuts ``pi . x >= pi0`` of the basic ``variables[t]`` (fractional part ``f0[t]``) of nodes
+        ``slots[t]`` of the previous simplex call, all in one launch (blp_simplex_gmi_cuts_host;
+        base_node.py:468-511 and floating_point.py:40). ``int_mask`` [n]: integer structurals.
+        Returns (pi [k, n], pi0 [k], code [k]) with code one of GMI_OK, GMI_NOT_BASIC, GMI_NONFINITE, GMI_ZERO."""
+        s = np.ascontiguousarray(slots, dtype=np.int32).ravel()
+        v = np.ascontiguousarray(variables, dtype=np.int32).ravel()
+        f = _f64(np.ravel(f0), (len(v),))
+        im = np.ascontiguousarray(int_mask, dtype=np.uint8).ravel()
+        if len(s) != len(v) or im.shape != (self.n,):
+            raise ValueError(f'need one slot per variable and an integer mask of length {self.n}')
+        k = len(v)
+        pi, pi0, code = np.empty((k, self.n)), np.empty(k), np.empty(k, dtype=np.int32)
+        _check(self._lib.blp_simplex_gmi_cuts_host(self._h, k, _np_ptr(s), _np_ptr(v), _np_ptr(f), _np_ptr(im),
+                                                   _np_ptr(pi), _np_ptr(pi0), _np_ptr(code)),
+               'blp_simplex_gmi_cuts_host')
+        return pi, pi0, code
+
     # -- device-buffer calls (torch tensors own the memory) --------------------------------------
     def solve_batch_device(self, lb, ub, row_mask=None, x0=None, y0=None, int_idx=None,
                            opts: Optional[BlpOpts] = None, want_x=True, want_y=True):
@@ -717,3 +739,6 @@ class MultiGpuBatchLP:
 
     def simplex_tableau_rows(self, slot: int, variables):
         raise BlpError('stored simplex factors are per device: MultiGpuBatchLP offers no tableau rows')
+
+    def simplex_gmi_cuts(self, slots, variables, f0, int_mask):
+        raise BlpError('stored simplex factors are per device: MultiGpuBatchLP offers no GMI cuts')

@@ -11,6 +11,7 @@ subclasses work unchanged. What differs is how the LP work is done:
 """
 from __future__ import annotations
 
+import copy
 import re
 import time
 from math import acos, ceil, degrees, floor
@@ -22,6 +23,7 @@ import scipy.sparse as sp
 import scipy.sparse.linalg as spla
 
 from simple_mip_solver_b200.compat.cylp_like import CyClpSimplex, CyLPArray, solve_lps
+from simple_mip_solver_b200.engine import GMI_OK, GMI_ZERO
 from simple_mip_solver_b200.utils.floating_point import numerically_safe_cut
 from simple_mip_solver_b200.utils.tolerance import (
     cutting_plane_progress_tolerance, good_coefficient_approximation_epsilon,
@@ -272,6 +274,14 @@ class BaseNode:
                                   cutting_plane_progress_tolerance, track_dual_bound: bool = False,
                                   **kwargs: Any) -> None:
         """One round: drop slack cuts, generate, select and append, re-solve (reference :292-324)."""
+        before = self._cut_round_prepare(cutting_plane_progress_tolerance, track_dual_bound, **kwargs)
+        self._bound_lp(track_dual_bound=track_dual_bound)
+        self._cut_round_finish(before, cutting_plane_progress_tolerance)
+
+    def _cut_round_prepare(self: T, cutting_plane_progress_tolerance: float = cutting_plane_progress_tolerance,
+                           track_dual_bound: bool = False, **kwargs: Any) -> float:
+        """First half of a cut round, up to the re-solve: returns the objective before it. Shared by
+        ``_cut_generation_iteration`` and the lock-step rounds of ``BranchAndBound(frontier_cut_rounds=True)``."""
         assert all(self.solution > -variable_epsilon), 'we must have x >= 0'
         assert isinstance(cutting_plane_progress_tolerance, float) and \
             cutting_plane_progress_tolerance > 0, 'cutting_plane_progress_tolerance must be positive'
@@ -284,7 +294,11 @@ class BaseNode:
         self._remove_slack_cuts(**kwargs)
         self.cut_pool = {**self.cut_pool, **self._generate_cuts(**kwargs)}
         self._select_cuts(**kwargs)
-        self._bound_lp(track_dual_bound=track_dual_bound)
+        return before
+
+    def _cut_round_finish(self: T, before: float,
+                          cutting_plane_progress_tolerance: float = cutting_plane_progress_tolerance) -> None:
+        """Second half of a cut round, after the re-solve: the stall test."""
         if before == 0 or abs(before - self.objective_value) / abs(before) < cutting_plane_progress_tolerance:
             self.cut_generation_stalled = True
             self.cut_generation_terminator = self.cut_generation_terminator or 'cuts not deep enough'
@@ -292,15 +306,17 @@ class BaseNode:
     def _remove_slack_cuts(self: T, **kwargs) -> List[str]:
         """Remove cut rows whose dual is zero (reference :326-341). A first-order dual is zero
         only up to the solve tolerance, so 'zero' means below 1e-9 of the largest row dual."""
-        duals = self.lp.dualConstraintSolution
-        biggest = max((float(np.max(np.abs(v))) for v in duals.values() if len(v)), default=0.0)
-        thresh = 1e-9 * max(1.0, biggest)
-        removable = [name for name, v in duals.items()
-                     if self.cut_name_pattern.match(name) and np.all(np.abs(v) <= thresh)]
+        removable = self._slack_cut_names()
         for name in removable:
             self.lp.removeConstraint(name)
         self._update_gmic_counts(cut_idxs=removable, operation='removed')
         return removable
+
+    def _slack_cut_names(self: T) -> List[str]:
+        duals = self.lp.dualConstraintSolution
+        biggest = max((float(np.max(np.abs(v))) for v in duals.values() if len(v)), default=0.0)
+        thresh = 1e-9 * max(1.0, biggest)
+        return [name for name, v in duals.items() if self.cut_name_pattern.match(name) and np.all(np.abs(v) <= thresh)]
 
     def _update_gmic_counts(self, cut_idxs: Union[Set[str], List[str], Dict[str, Any]],
                             operation: str) -> None:
@@ -316,18 +332,31 @@ class BaseNode:
         setattr(self, f'number_gmic_{operation}', getattr(self, f'number_gmic_{operation}') + hits)
 
     def _generate_cuts(self: T, gomory_cuts: bool = True, max_gomory_cuts: int = None,
-                       **kwargs) -> Dict[str, Tuple[CyLPArray, float]]:
+                       device_gomory: bool = False, **kwargs) -> Dict[str, Tuple[CyLPArray, float]]:
         """``max_gomory_cuts`` (new; default None = one cut per fractional basic integer variable, as
         the reference :365-385): only the rows of the most fractional ones — a root with thousands of
-        fractional variables would otherwise spend its time rounding thousands of dense cuts on the host."""
+        fractional variables would otherwise spend its time rounding thousands of dense cuts on the host.
+        ``device_gomory`` (new; default False): while the factorised basis of this LP's simplex solve is in
+        the engine's store, the cuts of the same rows are formed and rounded on the device in one call
+        (``_device_gomory_cuts``); their round-off is the device's, not the host's. Otherwise, and with the
+        option off, the host path."""
         assert isinstance(gomory_cuts, bool), 'gomory_cuts is boolean'
         assert max_gomory_cuts is None or (isinstance(max_gomory_cuts, int) and max_gomory_cuts > 0), \
             'max_gomory_cuts is a positive integer if provided'
+        assert isinstance(device_gomory, bool), 'device_gomory is boolean'
         pool = {}
         if gomory_cuts:
-            for row_idx, (pi, pi0) in self._find_gomory_cuts(max_rows=max_gomory_cuts).items():
-                name = f'cut_gomory_{self.idx}_{self.cut_generation_iterations}_{row_idx}'
-                pool[name] = numerically_safe_cut(pi=pi, pi0=pi0, estimate='over')
+            safe = None
+            if device_gomory:
+                safe = self.lp.memo_cuts(self.idx, self.cut_generation_iterations, max_gomory_cuts) \
+                    if self._status_override is None else None
+                if safe is None:
+                    safe = self._device_gomory_cuts(max_rows=max_gomory_cuts)
+            if safe is None:
+                safe = {row_idx: numerically_safe_cut(pi=pi, pi0=pi0, estimate='over')
+                        for row_idx, (pi, pi0) in self._find_gomory_cuts(max_rows=max_gomory_cuts).items()}
+            for row_idx, cut in safe.items():
+                pool[f'cut_gomory_{self.idx}_{self.cut_generation_iterations}_{row_idx}'] = cut
             self._update_gmic_counts(cut_idxs=pool, operation='created')
         return pool
 
@@ -410,7 +439,86 @@ class BaseNode:
         simplex kernels) the basis is the active set of the solution and is used only if the basic
         solution it defines reproduces the solver's x. Returns None when the status at hand
         (``_basis_status``) is not a basis of this solution."""
+        sel = self._gomory_rows(max_rows)
+        if sel is None:
+            return None
+        basic, wanted, is_basic, is_int, offset, sign, A, b = sel
         cuts = {}
+        if not wanted:
+            return cuts
+        n = self.lp.nVariables
+        rows = self._tableau_rows([int(basic[r]) for r, _ in wanted])
+        if rows is None:
+            return None
+        for (row_idx, f0), trow in zip(wanted, rows):
+            row = np.where(is_basic, 0.0, trow * sign)               # coefficients of the shifted nonbasics
+            f = row - np.floor(row)
+            pi_int = np.where(f <= f0, f / f0, (1 - f) / (1 - f0))
+            pi_cont = np.where(row > 0, row / f0, -row / (1 - f0))
+            pi_shift = np.where(is_int, pi_int, pi_cont)
+            pi_shift[is_basic] = 0.0
+            # sum pi' x' >= 1 with x'_j = sign_j (x_j - offset_j) for structurals, slack = A x - b
+            pi_x, pi_s = pi_shift[:n] * sign[:n], pi_shift[n:]
+            coefs = pi_x + A.T @ pi_s
+            rhs = 1.0 + float(np.dot(pi_x, offset[:n])) + float(np.dot(pi_s, b))
+            cuts[row_idx] = (CyLPArray(coefs), rhs)
+        return cuts
+
+    def _device_gomory_cuts(self: T, max_rows: int = None) -> Union[None, Dict[int, Tuple[CyLPArray, float]]]:
+        """The cuts ``_gomory_cuts_of_basis`` makes of the same rows, already rounded as
+        ``numerically_safe_cut(..., estimate='over')``, from ONE device call on the stored factor of this LP's
+        last simplex solve (``lp.gmi_cuts``, blp_simplex_gmi_cuts_host). None when that factor is gone, the
+        status at hand is not that solve's basis, or the device declines a row (a nonbasic column at an
+        infinite bound): the caller then takes the host path, which decides those cases as always."""
+        if self._status_override is not None:
+            return None
+        if not self.lp.has_stored_factor:
+            # with speculative cut rounds on, a solve the memo answered left no factor where the one-node-per-call
+            # run has one: solve it again (same start, same result) rather than take the host path
+            if not self.lp.restore_factor():
+                return None
+            if not getattr(self, '_speculative', False):
+                self.lp._shared.memo.cut_round_resolves += 1
+        req = self._gomory_requests(max_rows)
+        if req is None:
+            return None
+        if not req[0]:
+            return {}
+        got = self.lp.gmi_cuts(*req[1:])
+        return None if got is None else self._cuts_of_device(req[0], *got)
+
+    def _gomory_requests(self: T, max_rows: int = None):
+        """(wanted [(row position, f0)], basic variables, f0s, integer mask) of the rows ``_gomory_cuts_of_basis``
+        picks, or None when the status at hand is not a basis of this solution."""
+        sel = self._gomory_rows(max_rows)
+        if sel is None:
+            return None
+        basic, wanted = sel[0], sel[1]
+        int_mask = np.zeros(self.lp.nVariables, dtype=np.uint8)
+        int_mask[self._integer_indices] = 1
+        return wanted, [int(basic[r]) for r, _ in wanted], [f0 for _, f0 in wanted], int_mask
+
+    @staticmethod
+    def _cuts_of_device(wanted, pi, pi0, code) -> Union[None, Dict[int, Tuple[CyLPArray, float]]]:
+        """Cuts by row position from simplex_gmi_cuts' answer; None if the device declined a row."""
+        if not np.isin(code, (GMI_OK, GMI_ZERO)).all():
+            return None
+        return {row_idx: (CyLPArray(pi[t]), float(pi0[t])) for t, (row_idx, _) in enumerate(wanted)}
+
+    def _speculative_copy(self: T) -> T:
+        """A copy of this not yet bounded node for a speculative cut round (same idx, bounds, cuts, basis, cut
+        pool and last solve; its own LP object), so that no method of the real node runs."""
+        c = copy.copy(self)
+        c.lp = self.lp.clone()
+        c._cut_pool = dict(self._cut_pool)
+        c.cut_generation_dual_bound = dict(self.cut_generation_dual_bound)
+        c._speculative = True
+        return c
+
+    def _gomory_rows(self: T, max_rows: int = None):
+        """Which tableau rows ``_gomory_cuts_of_basis`` turns into cuts: (basic, wanted = [(row position, f0)],
+        is_basic, is_int, offset, sign over the n + m variables, A, b), or None when the status at hand is not a
+        basis of this solution."""
         n, m = self.lp.nVariables, self.lp.nConstraints
         col_stat, row_stat = self._basis_status()
         basic = self.basic_variable_indices
@@ -461,27 +569,10 @@ class BaseNode:
             if f0 < eps or f0 + eps > 1:
                 continue
             wanted.append((row_idx, f0))
-        if not wanted:
-            return cuts
         if max_rows is not None and len(wanted) > max_rows:
             keep = sorted(wanted, key=lambda t: -min(t[1], 1 - t[1]))[:max_rows]      # most fractional first (stable)
             wanted = sorted(keep)
-        rows = self._tableau_rows([int(basic[r]) for r, _ in wanted])
-        if rows is None:
-            return None
-        for (row_idx, f0), trow in zip(wanted, rows):
-            row = np.where(is_basic, 0.0, trow * sign)               # coefficients of the shifted nonbasics
-            f = row - np.floor(row)
-            pi_int = np.where(f <= f0, f / f0, (1 - f) / (1 - f0))
-            pi_cont = np.where(row > 0, row / f0, -row / (1 - f0))
-            pi_shift = np.where(is_int, pi_int, pi_cont)
-            pi_shift[is_basic] = 0.0
-            # sum pi' x' >= 1 with x'_j = sign_j (x_j - offset_j) for structurals, slack = A x - b
-            pi_x, pi_s = pi_shift[:n] * sign[:n], pi_shift[n:]
-            coefs = pi_x + A.T @ pi_s
-            rhs = 1.0 + float(np.dot(pi_x, offset[:n])) + float(np.dot(pi_s, b))
-            cuts[row_idx] = (CyLPArray(coefs), rhs)
-        return cuts
+        return basic, wanted, is_basic, is_int, offset, sign, A, b
 
     def _tableau_rows(self, variables: Sequence[int]):
         """Rows of inv([A, -I]_B) [A, -I] for the given basic variables: from the device when the
