@@ -4,8 +4,8 @@
 // blp_solve_batch runs restarted Halpern PDHG for a whole batch of node LPs:
 //   set-up kernels -> [ period graph: K x (k_primal, k_dual) | evaluation graph: k_tick,
 //   k_eval_cols, k_eval_rows, k_decide, k_apply_restart | harvest / refill of finished slots |
-//   wide batches: k_freeze_cols/rows (frozen flags per 32-node block), k_fold_cols/A/AT (the tiles'
-//   folded matrices), k_pow_A/AT/finish (step of the block that still moves), k_freeze_count ]
+//   wide batches: k_freeze_cols/rows (frozen flags per 32-node block), k_fold_cols, k_work_* (the tiles'
+//   work lists of the step kernels), k_pow_A/AT/finish (step of the block that still moves), k_freeze_count ]
 //   repeated until every node has a status -> output kernels.  The host reads 13 ints per period
 //   (nodes running / finished / restarting, frozen counts, watchdog resets).
 #include "../../include/blp.h"
@@ -466,16 +466,23 @@ size_t carve_state(const blp_handle h, int B, void* ws, DevState* S) {
     s.counters = cv.take<int32_t>(16);
     s.cfrz = cv.take<uint8_t>(n * (size_t)(ld / 32));
     s.rfrz = cv.take<uint8_t>(m * (size_t)(ld / 32));
-    {   // folded matrices of every 64-node tile (k_fold_*): 32 bytes per stored entry and tile
+    {   // folded matrices of every 64-node tile (k_fold_cols, k_work_*): 32 bytes per stored entry and tile
         const size_t tiles = ld / kBlk, nnz = h->A0.ptr.empty() ? 0 : (size_t)h->A0.ptr.back();
         s.cval = cv.take<double>(n * (size_t)(ld / 32));
         s.fcol = cv.take<uint8_t>(n * tiles);
         s.fval = cv.take<double>(n * tiles);
-        s.fentA = cv.take<Ent>(nnz * tiles);
-        s.fentAT = cv.take<Ent>(nnz * tiles);
-        s.fendA = cv.take<int32_t>(m * tiles);
-        s.fendAT = cv.take<int32_t>(n * tiles);
-        s.rconst = cv.take<double>(m * tiles);
+        auto work_list = [&](const size_t rows, const int rec_bytes) {
+            WorkList w;
+            w.row = cv.take<int2>((rows + 1) * tiles);
+            w.ent = cv.take<Ent>(nnz * tiles);
+            w.rec = cv.take<int4>(rows * tiles * (rec_bytes / 16));
+            w.chunk = cv.take<int4>(rows * tiles);
+            w.kept = cv.take<int32_t>(rows * tiles);
+            w.count = cv.take<int32_t>(tiles);
+            return w;
+        };
+        s.wlC = work_list(n, kPrimalRowBytes);
+        s.wlR = work_list(m, kDualRowBytes);
         s.ftc = cv.take<uint8_t>(n * tiles);
         s.ftr = cv.take<uint8_t>(m * tiles);
         s.pv = cv.take<double>(n * tiles);
@@ -524,7 +531,9 @@ struct StepArgs {
     double safety, cap;      // step of a tile = min(cap / ||A||, safety / ||A_UU||); safety 0 = keep 0.998 / ||A||
     int passes_first, passes;
 };
-int launch_freeze(const DevProb& P, const DevState& S, const FreezeArgs& F, const StepArgs& T, int mode, cudaStream_t st) {
+// pc / pr: the step plans, whose chunks the work lists are split over.
+int launch_freeze(const DevProb& P, const DevState& S, const FreezeArgs& F, const StepArgs& T, const Plan& pc,
+                  const Plan& pr, int mode, cudaStream_t st) {
     const int halves = (S.B + 31) / 32;
     auto rows_per_cta = [&](int rows) {
         const int want_chunks = std::max(1, 148 * 8 / halves);
@@ -537,9 +546,13 @@ int launch_freeze(const DevProb& P, const DevState& S, const FreezeArgs& F, cons
     const int tiles = (S.B + kBlk - 1) / kBlk;
     auto per_tile = [&](int rows) { return dim3(std::max(1, std::min((rows + kCtaThreads - 1) / kCtaThreads, 148 * 4 / tiles + 1)), tiles); };
     k_fold_cols<<<per_tile(P.n), kCtaThreads, 0, st>>>(P, S);
-    k_fold_A<<<per_tile(P.m), kCtaThreads, 0, st>>>(P, S);
-    k_fold_AT<<<per_tile(P.n), kCtaThreads, 0, st>>>(P, S);
-    int launched = 6;
+    k_work_count<true><<<per_tile(P.n), kCtaThreads, 0, st>>>(P, S);
+    k_work_count<false><<<per_tile(P.m), kCtaThreads, 0, st>>>(P, S);
+    k_work_scan<true><<<tiles, 1024, 0, st>>>(P, S, pc.chunks, pc.rows_per_cta);
+    k_work_scan<false><<<tiles, 1024, 0, st>>>(P, S, pr.chunks, pr.rows_per_cta);
+    k_work_fill<true><<<per_tile(P.n), kCtaThreads, 0, st>>>(P, S);
+    k_work_fill<false><<<per_tile(P.m), kCtaThreads, 0, st>>>(P, S);
+    int launched = 10;
     if (T.safety > 0.0) {
         const dim3 gp(std::min(kPowChunks, std::max(1, (std::max(P.n, P.m) + 4 * kCtaThreads - 1) / (4 * kCtaThreads))), tiles);
         if (mode == 2) k_pow_init<<<gp, kCtaThreads, 0, st>>>(P, S);
@@ -954,7 +967,7 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
     // frozen coordinates exist for the two-nodes-per-lane step kernels only (wide batches)
     auto refreeze = [&](int mode) {
         if (!freeze || pc.V != 2) return;
-        launches += launch_freeze(P, S, F, T, mode, st);
+        launches += launch_freeze(P, S, F, T, pc, pr, mode, st);
     };
     refreeze(2);
 
@@ -1043,7 +1056,7 @@ int blp_solve_batch(blp_handle h, int B, const double* lb, const double* ub,
                     // the slots moved: the tiles are new sets of nodes and their flags start afresh (x', y' travelled
                     // with the nodes); a batch that has become too narrow for the freezing kernels updates every
                     // coordinate again, so its nodes return to the step of the full matrix
-                    if (pc.V == 2) launches += launch_freeze(P, S, F, T, 2, st);
+                    if (pc.V == 2) launches += launch_freeze(P, S, F, T, pc, pr, 2, st);
                     else k_eta_reset<<<(S.ld + 127) / 128, 128, 0, st>>>(P, S), ++launches;
                 }
                 coop_rejected = false;

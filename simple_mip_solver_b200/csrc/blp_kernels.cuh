@@ -71,6 +71,20 @@ struct DevProb {
     double bcut2;          // sum of squares of the (unscaled) right-hand sides of ALL appended rows
 };
 
+// Work list of a frozen-path step kernel for every 64-node tile (k_work_*, rebuilt once per evaluation period): the
+// rows that are not frozen for the tile (ACTIVE rows), those of more than kLongRow stored entries first, then the
+// others, each group in ascending row order; their kept entries packed in that order; one record of row scalars per
+// active row; and one header per (tile, chunk) of the launch grid. Rows of the step kernel: columns of A (primal,
+// rows = n) or rows of A (dual, rows = m).
+struct WorkList {
+    int2* row;       // [tile][rows + 1] active row k: {row id, start of its entries in ent}; k = count: {-1, end}
+    Ent* ent;        // [tile][nnz]
+    int4* rec;       // [tile][rows][kPrimalRowBytes / 16 or kDualRowBytes / 16] row scalars (primal_rec / dual_rec)
+    int4* chunk;     // [tile][rows] chunk header {first active row, rows (-1: one long row), first entry, end entry}
+    int32_t* kept;   // [tile][rows] kept entries of a row, -1 = frozen (k_work_count; k_work_scan's scratch)
+    int32_t* count;  // [tile] active rows
+};
+
 struct DevState {
     int B, ld;
     double *xbar, *l, *u, *X1, *DX, *G;            // [n][ld]
@@ -95,14 +109,12 @@ struct DevState {
     // Frozen coordinates (k_freeze_cols / k_freeze_rows): one byte per (32-node block, row), layout
     // [block][row] like lref; 1 = every running node of the block agrees that the coordinate rests.
     uint8_t *cfrz, *rfrz;
-    // Folded matrices of a 64-node tile (k_fold_*): the entries the step kernels still have to gather once the
-    // frozen coordinates are taken out. Row i of tile t keeps its slots [ptr[i], ptr[i+1]) in a per-tile copy of the
-    // entry array, the kept entries packed to the front; fendA / fendAT hold the end of the kept part.
+    // Folded matrices of a 64-node tile: the entries the step kernels still have to gather once the frozen
+    // coordinates are taken out, as work lists (k_work_*). A folded column's contribution to a row of A is summed
+    // into the row's rconst (the dual record's second scalar) once per evaluation period.
     double* cval;                                  // [block][n] x' of a frozen column if the block's nodes agree on it
     uint8_t* fcol; double* fval;                   // [tile][n] column folded into rconst, with the value it rests at
-    Ent *fentA, *fentAT;                           // [tile][nnz]
-    int32_t *fendA, *fendAT;                       // [tile][m], [tile][n]
-    double* rconst;                                // [tile][m] sum of a_ij x_j over the folded columns of row i
+    WorkList wlC, wlR;                             // primal step (rows of A'), dual step (rows of A)
     // Step size of a node (k_pow_*): eta = P.eta = 0.998 / ||A|| unless its tile has frozen coordinates, then up to
     // safety / ||A_UU||, A_UU = the rows and columns of the tile that still move.
     double* eta; int32_t* eta_lock;                // [ld] current step; 1 = the watchdog sent the node back to P.eta
@@ -222,7 +234,6 @@ struct Slab {
     const int* sp;       // shared: absolute row pointers of rows r0 .. r1
     const int4* se;      // shared: entries [sp[0], sp[nrows]) or nullptr if they did not fit
     int base;
-    const int* ends = nullptr;   // shared: end of row lr's entries if it is not sp[lr + 1] (folded matrices)
 };
 
 extern __shared__ int4 dyn_smem[];
@@ -575,7 +586,7 @@ __device__ __forceinline__ void dot2_entries(const int4* __restrict__ E, const i
 __device__ __forceinline__ void slab_dot2(const Slab& sl, const Ent* __restrict__ ent, const int lr,
                                           const double* __restrict__ Vn, double& g0, double& g1,
                                           const int ld = kBlk) {
-    const int p0 = sl.sp[lr], p1 = sl.ends ? sl.ends[lr] : sl.sp[lr + 1];
+    const int p0 = sl.sp[lr], p1 = sl.sp[lr + 1];
     if (sl.se) dot2_entries<true>(sl.se - sl.base, p0, p1, Vn, g0, g1, ld);
     else dot2_entries<false>(reinterpret_cast<const int4*>(ent), p0, p1, Vn, g0, g1, ld);
 }
@@ -583,11 +594,10 @@ __device__ __forceinline__ void slab_dot2(const Slab& sl, const Ent* __restrict_
 // A chunk that consists of ONE long row (a dense cut row, typically) is shared by all warps of the
 // CTA: each warp gathers a slice of the row's entries, the partial sums meet in shared memory.
 
-__device__ __forceinline__ void coop_dot2(const Slab& sl, const Ent* __restrict__ ent,
+__device__ __forceinline__ void coop_dot2(const Slab& sl, const Ent* __restrict__ ent, const int p0, const int p1,
                                           const double* __restrict__ Vn, const int warp, const int lane,
                                           double& g0, double& g1) {
     __shared__ double2 red[kWarps][32];
-    const int p0 = sl.sp[0], p1 = sl.ends ? sl.ends[0] : sl.sp[1];
     const int seg = ((p1 - p0 + kWarps - 1) / kWarps + BLP_U - 1) / BLP_U * BLP_U;
     const int a = min(p1, p0 + warp * seg), b = min(p1, a + seg);
     double s0 = 0.0, s1 = 0.0;
@@ -604,81 +614,10 @@ __device__ __forceinline__ void coop_dot2(const Slab& sl, const Ent* __restrict_
     }
 }
 
-// Frozen coordinates of a CTA's chunk (rows [r0, r1) of the node tile whose 32-node blocks are h0, h0 + 1): one
-// byte per row in shared memory, 1 = both blocks agree (a block without a running node agrees to everything).
-// `live` is the warp's ballot of running lanes: lanes 0-15 hold the nodes of block h0, lanes 16-31 those of h0 + 1.
+// Rows of a frozen-path CTA's chunk as in its work list, {row id, start of its entries} (stage_work): a trip reads
+// both with one 64-bit load, and the end of its entries from the next row.
 constexpr int kMaxChunkRows = 512;
-__shared__ uint16_t s_rows[kMaxChunkRows];   // local rows of the chunk that are NOT frozen, ascending
-__shared__ int s_ends[kMaxChunkRows];        // end of the kept entries of each local row (folded matrix)
-__shared__ int s_group[kMaxChunkRows / 32 + 1];
-__shared__ int s_nrows;
-
-// Slab of a CTA whose tile has frozen coordinates: as stage_slab, plus the CTA's WORK LIST — the rows of its chunk
-// that are not frozen for this tile (both 32-node blocks h0, h0 + 1 agree, a block without a running node agrees to
-// everything), compacted so the warps share them evenly — and the ends of the rows' kept entries in the tile's
-// folded matrix `ent`. Everything global is loaded in the two phases stage_slab has anyway (pointers, ends and
-// flags together, then the entries), so a CTA pays no extra round trip. `live`: the warp's ballot of running lanes,
-// lanes 0-15 hold the nodes of block h0, lanes 16-31 those of h0 + 1. `rs`: per-row scalars of the work-list rows,
-// loaded in phase 2 with the entries.
-template <class RS>
-__device__ __forceinline__ Slab stage_slab_frozen(const int32_t* __restrict__ ptr, const Ent* __restrict__ ent,
-                                                  const int32_t* __restrict__ ends, const uint8_t* __restrict__ flags,
-                                                  const int rows, const int h0, const unsigned live, const int r0,
-                                                  const int r1, const int rows_per_cta, const int cap, const RS rs) {
-    int* sp = reinterpret_cast<int*>(dyn_smem);
-    int4* se = dyn_smem + (rows_per_cta + 4) / 4;
-    const int nrows = r1 - r0, lane = threadIdx.x & 31;
-    const bool live0 = (live & 0x0000ffffu) != 0, live1 = (live & 0xffff0000u) != 0;
-    const uint8_t* __restrict__ f0 = flags + (size_t)h0 * rows + r0;
-    const uint8_t* __restrict__ f1 = f0 + rows;
-    // phase 1: row pointers, row ends, flags; a thread owns local rows t and t + 256
-    bool keep[2];
-    int rank[2];
-#pragma unroll
-    for (int q = 0; q < 2; ++q) {
-        const int t = threadIdx.x + q * kCtaThreads;
-        keep[q] = false;
-        if (t <= nrows) sp[t] = __ldg(ptr + r0 + t);
-        if (t < nrows) {
-            s_ends[t] = __ldg(ends + r0 + t);
-            keep[q] = !((!live0 || f0[t] != 0) && (!live1 || f1[t] != 0));
-        }
-        const unsigned bal = __ballot_sync(0xffffffffu, keep[q]);
-        rank[q] = __popc(bal & ((1u << lane) - 1u));
-        if (lane == 0) s_group[t >> 5] = __popc(bal);
-    }
-    __syncthreads();
-    Slab s;
-    s.sp = sp;
-    s.base = sp[0];
-    s.se = nullptr;
-    s.ends = s_ends;
-    const int cnt = sp[nrows] - s.base;
-    // phase 2: the entries (their loads fly while the work list is written)
-    if (cnt <= cap) {
-        const int4* __restrict__ src = reinterpret_cast<const int4*>(ent) + s.base;
-        for (int t = threadIdx.x; t < cnt; t += kCtaThreads) se[t] = __ldg(src + t);
-        s.se = se;
-    }
-    const int groups = (nrows + 31) >> 5;
-#pragma unroll
-    for (int q = 0; q < 2; ++q) {
-        const int t = threadIdx.x + q * kCtaThreads;
-        if (keep[q]) {
-            int before = 0;
-            for (int g = 0; g < (t >> 5); ++g) before += s_group[g];
-            s_rows[before + rank[q]] = (uint16_t)t;
-            rs(r0 + t, before + rank[q]);
-        }
-    }
-    if (threadIdx.x == 0) {
-        int total = 0;
-        for (int g = 0; g < groups; ++g) total += s_group[g];
-        s_nrows = total;
-    }
-    __syncthreads();
-    return s;
-}
+__shared__ int2 s_row[kMaxChunkRows + 1];
 
 // What a warp's trip over one row reads besides the row's state and gathers, staged with the slab (no round trip of
 // its own) and read from shared memory after the gathers are issued. At 48 registers (5 CTAs per SM) the compiler
@@ -695,59 +634,103 @@ __device__ __forceinline__ int4* row_scalar_smem(const int rows_per_cta, const i
 // Bytes per chunk row (host side sizes the launch with them).
 constexpr int kPrimalRowBytes = 48, kDualRowBytes = 16;
 
-// primal step: c_j, and (lref, uref), lumask of row j in the tile's two 32-node blocks h0, h0 + 1
+// One record of row scalars per chunk row, the same in shared memory and in a work list (WorkList::rec).
+// primal step: (lref, uref) of row j in the tile's two 32-node blocks h0, h0 + 1, c_j, and the blocks' lumask words
+struct PrimalRec {
+    double2 lu[2];
+    double c;
+    uint32_t mk[2];
+};
+// dual step: b_i, and rconst of row i in the tile (frozen coordinates) or 0
+struct DualRec {
+    double b, rc;
+};
+static_assert(sizeof(PrimalRec) == kPrimalRowBytes && sizeof(DualRec) == kDualRowBytes, "row record sizes");
+
+// rs(j, slot) of stage_slab: loads the primal record of row j, stores it at rec[slot]
 struct PrimalRowScalars {
     const double* c; const double* lref; const double* uref; const uint32_t* lumask;   // at block h0
     size_t rows;                                                                    // block stride
-    // the staged arrays; a trip rebuilds this from the kernel parameters instead of keeping pointers in registers
-    struct View {
-        double2* lu; double* cs; uint32_t* mk;                                      // [slot][2], [slot], [slot][2]
-        __device__ __forceinline__ View(const int rows_per_cta, const int cap) {
-            lu = reinterpret_cast<double2*>(row_scalar_smem(rows_per_cta, cap));
-            cs = reinterpret_cast<double*>(lu + 2 * rows_per_cta);
-            mk = reinterpret_cast<uint32_t*>(cs + rows_per_cta);
-        }
-    };
-    View v;
-    __device__ PrimalRowScalars(const DevProb& P, const DevState& S, const int h0, const int rows_per_cta,
-                                const int cap) : v(rows_per_cta, cap) {
+    PrimalRec* rec;
+    __device__ PrimalRowScalars(const DevProb& P, const DevState& S, const int h0, PrimalRec* dst) : rec(dst) {
         const size_t f = (size_t)h0 * P.n;
         c = P.c; lref = S.lref + f; uref = S.uref + f; lumask = S.lumask + f; rows = P.n;
     }
     __device__ __forceinline__ void operator()(const int j, const int slot) const {
-        v.cs[slot] = __ldg(c + j);
-        v.lu[2 * slot] = make_double2(__ldg(lref + j), __ldg(uref + j));
-        v.lu[2 * slot + 1] = make_double2(__ldg(lref + rows + j), __ldg(uref + rows + j));
-        v.mk[2 * slot] = __ldg(lumask + j);
-        v.mk[2 * slot + 1] = __ldg(lumask + rows + j);
+        PrimalRec r;
+        r.lu[0] = make_double2(__ldg(lref + j), __ldg(uref + j));
+        r.lu[1] = make_double2(__ldg(lref + rows + j), __ldg(uref + rows + j));
+        r.c = __ldg(c + j);
+        r.mk[0] = __ldg(lumask + j);
+        r.mk[1] = __ldg(lumask + rows + j);
+        rec[slot] = r;
     }
 };
 
-// dual step: b_i, and rconst of row i in the tile (frozen coordinates) or 0
+// the same for the dual step without frozen coordinates (rconst 0)
 struct DualRowScalars {
-    const double* b; const double* rc;      // rc: null without frozen coordinates
-    struct View {
-        double* bs; double* rcs;            // [slot], [slot]
-        __device__ __forceinline__ View(const int rows_per_cta, const int cap) {
-            bs = reinterpret_cast<double*>(row_scalar_smem(rows_per_cta, cap));
-            rcs = bs + rows_per_cta;
-        }
-    };
-    View v;
-    __device__ DualRowScalars(const DevProb& P, const double* rconst, const int rows_per_cta, const int cap)
-        : b(P.b), rc(rconst), v(rows_per_cta, cap) {}
-    __device__ __forceinline__ void operator()(const int i, const int slot) const {
-        v.bs[slot] = __ldg(b + i);
-        v.rcs[slot] = rc ? __ldg(rc + i) : 0.0;
-    }
+    const double* b;
+    DualRec* rec;
+    __device__ __forceinline__ void operator()(const int i, const int slot) const { rec[slot] = DualRec{__ldg(b + i), 0.0}; }
 };
 
+// Slab of a frozen-path CTA: chunk `hd` of its tile's work list W (k_work_scan). Every address is known from the
+// header, so the chunk's rows (s_row), its row records (row_scalar_smem) and, when they fit in `cap`, its kept entries
+// are copied in one round trip. The slab has no row pointers: a trip finds its entries through s_row.
+template <class Rec>
+__device__ __forceinline__ Slab stage_work(const WorkList& W, const int rows, const int nnz, const int tile,
+                                           const int4 hd, const int rows_per_cta, const int cap) {
+    constexpr int RQ = sizeof(Rec) / sizeof(int4);
+    int4* se = dyn_smem + (rows_per_cta + 4) / 4;
+    int4* sr = row_scalar_smem(rows_per_cta, cap);
+    const int nk = hd.y < 0 ? 1 : hd.y, cnt = hd.w - hd.z;
+    const bool fits = cnt <= cap;
+    const int2* __restrict__ rw = W.row + (size_t)tile * (rows + 1) + hd.x;
+    const int4* __restrict__ rr = W.rec + ((size_t)tile * rows + hd.x) * RQ;
+    const int4* __restrict__ re = reinterpret_cast<const int4*>(W.ent + (size_t)tile * nnz) + hd.z;
+    const int units = max(max(nk + 1, nk * RQ), fits ? cnt : 0);
+    for (int t0 = threadIdx.x; t0 < units; t0 += 2 * kCtaThreads) {
+        int2 r[2];
+        int4 s[2], e[2];
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {                          // all loads first, then the stores
+            const int t = t0 + q * kCtaThreads;
+            if (t <= nk) r[q] = __ldg(rw + t);
+            if (t < nk * RQ) s[q] = __ldg(rr + t);
+            if (fits && t < cnt) e[q] = __ldg(re + t);
+        }
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const int t = t0 + q * kCtaThreads;
+            if (t <= nk) s_row[t] = r[q];
+            if (t < nk * RQ) sr[t] = s[q];
+            if (fits && t < cnt) se[t] = e[q];
+        }
+    }
+    __syncthreads();
+    Slab s;
+    s.sp = nullptr;
+    s.base = hd.z;
+    s.se = fits ? se : nullptr;
+    return s;
+}
+
+// Frozen-path CTAs (iterations 0 .. K-2 of a period with frozen coordinates) walk a chunk of their tile's work list:
+// its active rows only, each with its kept entries. The last iteration of a period (MAJOR) and batches without
+// frozen coordinates walk rows [r0, r1) of the full matrix (chunk_ptr).
 template <bool MAJOR>
 __global__ void __launch_bounds__(kCtaThreads, BLP_MINB2)
 k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_cta, const int cap,
           const int* __restrict__ chunk_ptr, const int tile0) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int node = (tile0 + blockIdx.y) * kBlk + lane * 2;   // this lane: nodes node, node + 1
+    const int tile = tile0 + blockIdx.y;
+    const int node = tile * kBlk + lane * 2;                   // this lane: nodes node, node + 1
+    const bool frz = !MAJOR && S.cfrz != nullptr;
+    // the chunk header and the nodes' scalars are loaded together: one round trip
+    const int4 hd = frz ? __ldg(S.wlC.chunk + (size_t)tile * P.n + blockIdx.x)
+                        : make_int4(__ldg(chunk_ptr + 2 * blockIdx.x), __ldg(chunk_ptr + 2 * blockIdx.x + 1), 0, 0);
+    const int2 sb = *reinterpret_cast<const int2*>(S.sbase + node);
+    const double2 et = ld2(S.eta + node), om = ld2(S.omega + node);
     const bool k0 = node < S.B && S.fin[node] == 0;
     const bool k1 = node + 1 < S.B && S.fin[node + 1] == 0;
     const unsigned live = __ballot_sync(0xffffffffu, k0 || k1);
@@ -757,56 +740,48 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
     const unsigned run0 = __ballot_sync(0xffffffffu, k0), run1 = __ballot_sync(0xffffffffu, k1);
     auto st0 = [&] { return MAJOR ? k0 : ((run0 >> (threadIdx.x & 31)) & 1u) != 0; };
     auto st1 = [&] { return MAJOR ? k1 : ((run1 >> (threadIdx.x & 31)) & 1u) != 0; };
-    double w0 = 0, w1 = 0, tau0 = 0, tau1 = 0;
-    if (k0) {
-        const int s = S.sbase[node] + it;
-        w0 = (double)s / (double)(s + 1);
-        tau0 = S.eta[node] / S.omega[node];
-    }
-    if (k1) {
-        const int s = S.sbase[node + 1] + it;
-        w1 = (double)s / (double)(s + 1);
-        tau1 = S.eta[node + 1] / S.omega[node + 1];
-    }
     if (warp == 0) {                                           // every warp has the same; read back after the stage
-        s_wv[lane] = make_double2(w0, w1);
-        s_sv[lane] = make_double2(tau0, tau1);
+        const int s0 = sb.x + it, s1 = sb.y + it;
+        s_wv[lane] = make_double2(k0 ? (double)s0 / (double)(s0 + 1) : 0.0, k1 ? (double)s1 / (double)(s1 + 1) : 0.0);
+        s_sv[lane] = make_double2(k0 ? et.x / om.x : 0.0, k1 ? et.y / om.y : 0.0);
     }
-    const int r0 = __ldg(chunk_ptr + 2 * blockIdx.x);
-    const int r1 = __ldg(chunk_ptr + 2 * blockIdx.x + 1);
-    const bool frz = !MAJOR && S.cfrz != nullptr;
-    const int tile = tile0 + blockIdx.y;
-    // with frozen coordinates: the tile's folded A' (entries of frozen rows, whose multiplier is zero, taken out)
-    const Ent* __restrict__ cent = frz ? S.fentAT + (size_t)tile * P.nnz : P.cent;
-    const PrimalRowScalars rs(P, S, tile * 2, rows_per_cta, cap);
-    const Slab sl = frz ? stage_slab_frozen(P.cptr, cent, S.fendAT + (size_t)tile * P.n, S.cfrz, P.n, tile * 2, live,
-                                            r0, r1, rows_per_cta, cap, rs)
-                        : stage_slab(P.cptr, P.cent, r0, r1, rows_per_cta, cap, dyn_smem, rs);
+    if (frz && hd.y == 0) return;                              // no active row left for this chunk
+    const int r0 = hd.x, r1 = hd.y;                            // rows of the full matrix (not frz)
+    // with frozen coordinates: the tile's kept entries of A' (entries of frozen rows, whose multiplier is zero, taken out)
+    const Ent* __restrict__ cent = frz ? S.wlC.ent + (size_t)tile * P.nnz : P.cent;
+    PrimalRec* const recs = reinterpret_cast<PrimalRec*>(row_scalar_smem(rows_per_cta, cap));
+    const Slab sl = frz ? stage_work<PrimalRec>(S.wlC, P.n, P.nnz, tile, hd, rows_per_cta, cap)
+                        : stage_slab(P.cptr, P.cent, r0, r1, rows_per_cta, cap, dyn_smem,
+                                     PrimalRowScalars(P, S, tile * 2, recs));
     // 32-bit element indices: the host picks these kernels only for state arrays of fewer than 2^32 elements
     const unsigned base = (unsigned)tix(0, node, P.n);
     const double* __restrict__ yn = S.y + tix(0, node, P.m);
     const unsigned yoff = (unsigned)tix(0, node, P.m);
     const unsigned bit = node & 31;
     const int half = lane >> 4;                                // lanes 16-31: nodes of block h0 + 1
-    const bool coop = (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
+    const bool coop = frz ? hd.y < 0 : (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
+    // row slot k of the chunk: {row, start of its entries}; its entries end where row k + 1's start
+    auto row_at = [&](const int k) { return frz ? s_row[k] : make_int2(r0 + k, sl.sp[k]); };
     double cg0 = 0.0, cg1 = 0.0;
+    int2 rc = make_int2(0, 0);
     if (coop) {
-        if (frz && s_nrows == 0) return;
-        coop_dot2(sl, cent, yn, warp, lane, cg0, cg1);
+        rc = row_at(0);
+        coop_dot2(sl, cent, rc.y, row_at(1).y, yn, warp, lane, cg0, cg1);
         if (warp != 0) return;
     }
-    // one warp trip: row slot k of the work list; gather(lr, g0, g1) adds the row's gather-dot to (g0, g1)
-    auto trip = [&](const int k, double g0, double g1, auto gather) {
-        const int lr = frz ? (int)s_rows[k] : k;
-        const unsigned e = base + (unsigned)(r0 + lr) * kBlk;
+    // one warp trip: row slot k of the chunk (rk = row_at(k)); gather(p0, p1, g0, g1) adds the gather-dot of entries
+    // [p0, p1) to (g0, g1)
+    auto trip = [&](const int k, const int2 rk, double g0, double g1, auto gather) {
+        const int p1 = row_at(k + 1).y;
+        const unsigned e = base + (unsigned)rk.x * kBlk;
         const double2 xb = ld2(S.xbar + e);
         const double2 a = ldcs2(S.xa + e);
-        gather(lr, g0, g1);
+        gather(rk.y, p1, g0, g1);
         // the rest of the row's inputs come from shared memory once the gathers fly; the dense bounds of nodes
         // that deviate from their block's reference (about 1 % of rows) only after them
-        const PrimalRowScalars::View rv(rows_per_cta, cap);
-        const uint32_t mk = (rv.mk[2 * k + half] >> bit) & 3u;
-        const double2 lh = rv.lu[2 * k + half];
+        const PrimalRec* rv = reinterpret_cast<const PrimalRec*>(row_scalar_smem(rows_per_cta, cap)) + k;
+        const uint32_t mk = (rv->mk[half] >> bit) & 3u;
+        const double2 lh = rv->lu[half];
         double lo0 = lh.x, hi0 = lh.y, lo1 = lh.x, hi1 = lh.y;
         if (mk & 1u) {                                         // node deviates from its block's reference
             lo0 = __ldcs(S.l + e);
@@ -816,7 +791,7 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
             lo1 = __ldcs(S.l + e + 1);
             hi1 = __ldcs(S.u + e + 1);
         }
-        const double cj = rv.cs[k];
+        const double cj = rv->c;
         const double2 w = s_wv[lane], tau = s_sv[lane];
         const double xc0 = fma(w.x, xb.x - a.x, a.x), xc1 = fma(w.y, xb.y - a.y, a.y);
         const double xp0 = fmin(fmax(xc0 - tau.x * (cj - g0), lo0), hi0);
@@ -829,23 +804,23 @@ k_primal2(const DevProb P, const DevState S, const int it, const int rows_per_ct
         }
     };
     if (coop) {                                                // warp 0, the chunk's one row
-        trip(0, cg0, cg1, [](int, double&, double&) {});
+        trip(0, rc, cg0, cg1, [](int, int, double&, double&) {});
         return;
     }
     // Whether the entries sit in shared memory is the same for the whole CTA: choosing the loop here keeps the
     // choice (and its pointer) out of the registers that are live across a trip's gathers.
-    const int ntrips = frz ? s_nrows : r1 - r0;                // frozen columns rest at their bound for the whole tile
+    const int ntrips = frz ? hd.y : r1 - r0;                   // frozen columns rest at their bound for the whole tile
     if (sl.se) {
         const int4* const E = sl.se - sl.base;
         for (int k = warp; k < ntrips; k += kWarps)
-            trip(k, 0.0, 0.0, [&](const int lr, double& g0, double& g1) {
-                dot2_entries<true, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.y, g0, g1, kBlk, yoff);
+            trip(k, row_at(k), 0.0, 0.0, [&](const int p0, const int p1, double& g0, double& g1) {
+                dot2_entries<true, unsigned, false>(E, p0, p1, S.y, g0, g1, kBlk, yoff);
             });
     } else {
         const int4* const E = reinterpret_cast<const int4*>(cent);
         for (int k = warp; k < ntrips; k += kWarps)
-            trip(k, 0.0, 0.0, [&](const int lr, double& g0, double& g1) {
-                dot2_entries<false, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.y, g0, g1, kBlk, yoff);
+            trip(k, row_at(k), 0.0, 0.0, [&](const int p0, const int p1, double& g0, double& g1) {
+                dot2_entries<false, unsigned, false>(E, p0, p1, S.y, g0, g1, kBlk, yoff);
             });
     }
 }
@@ -855,7 +830,13 @@ __global__ void __launch_bounds__(kCtaThreads, BLP_MINB2)
 k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta, const int cap,
         const int* __restrict__ chunk_ptr, const int tile0) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int node = (tile0 + blockIdx.y) * kBlk + lane * 2;
+    const int tile = tile0 + blockIdx.y;
+    const int node = tile * kBlk + lane * 2;
+    const bool frz = !MAJOR && S.rfrz != nullptr;
+    const int4 hd = frz ? __ldg(S.wlR.chunk + (size_t)tile * P.m + blockIdx.x)     // as in k_primal2
+                        : make_int4(__ldg(chunk_ptr + 2 * blockIdx.x), __ldg(chunk_ptr + 2 * blockIdx.x + 1), 0, 0);
+    const int2 sb = *reinterpret_cast<const int2*>(S.sbase + node);
+    const double2 et = ld2(S.eta + node), om = ld2(S.omega + node);
     const bool k0 = node < S.B && S.fin[node] == 0;
     const bool k1 = node + 1 < S.B && S.fin[node + 1] == 0;
     const unsigned live = __ballot_sync(0xffffffffu, k0 || k1);
@@ -863,52 +844,42 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
     const unsigned run0 = __ballot_sync(0xffffffffu, k0), run1 = __ballot_sync(0xffffffffu, k1);   // as in k_primal2
     auto st0 = [&] { return ((run0 >> (threadIdx.x & 31)) & 1u) != 0; };
     auto st1 = [&] { return ((run1 >> (threadIdx.x & 31)) & 1u) != 0; };
-    double w0 = 0, w1 = 0, sig0 = 0, sig1 = 0;
-    if (k0) {
-        const int s = S.sbase[node] + it;
-        w0 = (double)(s + 1) / (double)(s + 2);
-        sig0 = S.eta[node] * S.omega[node];
-    }
-    if (k1) {
-        const int s = S.sbase[node + 1] + it;
-        w1 = (double)(s + 1) / (double)(s + 2);
-        sig1 = S.eta[node + 1] * S.omega[node + 1];
-    }
     if (warp == 0) {                                           // every warp has the same; read back after the stage
-        s_wv[lane] = make_double2(w0, w1);
-        s_sv[lane] = make_double2(sig0, sig1);
+        const int s0 = sb.x + it, s1 = sb.y + it;
+        s_wv[lane] = make_double2(k0 ? (double)(s0 + 1) / (double)(s0 + 2) : 0.0,
+                                  k1 ? (double)(s1 + 1) / (double)(s1 + 2) : 0.0);
+        s_sv[lane] = make_double2(k0 ? et.x * om.x : 0.0, k1 ? et.y * om.y : 0.0);
     }
-    const int r0 = __ldg(chunk_ptr + 2 * blockIdx.x);
-    const int r1 = __ldg(chunk_ptr + 2 * blockIdx.x + 1);
-    const bool frz = !MAJOR && S.rfrz != nullptr;
-    const int tile = tile0 + blockIdx.y;
-    // with frozen coordinates: the tile's folded A (columns that rest at one value for the whole tile are summed
-    // into rconst once per evaluation period instead of being gathered every iteration)
-    const Ent* __restrict__ aent = frz ? S.fentA + (size_t)tile * P.nnz : P.ent;
-    const double* __restrict__ rconst = S.rconst + (size_t)tile * P.m;
-    const DualRowScalars rs(P, frz ? rconst : nullptr, rows_per_cta, cap);
-    const Slab sl = frz ? stage_slab_frozen(P.rowptr, aent, S.fendA + (size_t)tile * P.m, S.rfrz, P.m, tile * 2, live,
-                                            r0, r1, rows_per_cta, cap, rs)
-                        : stage_slab(P.rowptr, P.ent, r0, r1, rows_per_cta, cap, dyn_smem, rs);
+    if (frz && hd.y == 0) return;
+    const int r0 = hd.x, r1 = hd.y;
+    // with frozen coordinates: the tile's kept entries of A (columns that rest at one value for the whole tile are
+    // summed into the row's rconst once per evaluation period instead of being gathered every iteration)
+    const Ent* __restrict__ aent = frz ? S.wlR.ent + (size_t)tile * P.nnz : P.ent;
+    DualRec* const recs = reinterpret_cast<DualRec*>(row_scalar_smem(rows_per_cta, cap));
+    const Slab sl = frz ? stage_work<DualRec>(S.wlR, P.m, P.nnz, tile, hd, rows_per_cta, cap)
+                        : stage_slab(P.rowptr, P.ent, r0, r1, rows_per_cta, cap, dyn_smem, DualRowScalars{P.b, recs});
     const unsigned base = (unsigned)tix(0, node, P.m);      // 32-bit element indices, as in k_primal2
     const double* __restrict__ xn = S.xbar + tix(0, node, P.n);
     const unsigned xoff = (unsigned)tix(0, node, P.n);
-    const bool coop = (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
+    const bool coop = frz ? hd.y < 0 : (r1 - r0 == 1) && (sl.sp[1] - sl.sp[0] > kLongRow);
+    auto row_at = [&](const int k) { return frz ? s_row[k] : make_int2(r0 + k, sl.sp[k]); };   // as in k_primal2
     double cg0 = 0.0, cg1 = 0.0;
+    int2 rc = make_int2(0, 0);
     if (coop) {
-        if (frz && s_nrows == 0) return;
-        coop_dot2(sl, aent, xn, warp, lane, cg0, cg1);
+        rc = row_at(0);
+        coop_dot2(sl, aent, rc.y, row_at(1).y, xn, warp, lane, cg0, cg1);
         if (warp != 0) return;
         if (frz) {
-            const double rc = __ldg(rconst + r0);
+            const double rc = recs[0].rc;
             cg0 += rc;
             cg1 += rc;
         }
     }
-    // one warp trip: row slot k of the work list; gather(k, lr, ax0, ax1) sets (ax0, ax1) to the row's A x
-    auto trip = [&](const int k, auto gather) {
-        const int lr = frz ? (int)s_rows[k] : k;
-        const int i = r0 + lr;
+    // one warp trip: row slot k of the chunk (rk = row_at(k)); gather(k, p0, p1, ax0, ax1) sets (ax0, ax1) to the
+    // row's A x
+    auto trip = [&](const int k, const int2 rk, auto gather) {
+        const int p1 = row_at(k + 1).y;
+        const int i = rk.x;
         const unsigned e = base + (unsigned)i * kBlk;
         const double2 yc = ld2(S.y + e);
         const double2 a = ldcs2(S.ya + e);
@@ -919,8 +890,8 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
             on1 = mrow[1] != 0;
         }
         double ax0, ax1;
-        gather(k, lr, ax0, ax1);
-        const double bi = DualRowScalars::View(rows_per_cta, cap).bs[k];
+        gather(k, rk.y, p1, ax0, ax1);
+        const double bi = reinterpret_cast<const DualRec*>(row_scalar_smem(rows_per_cta, cap))[k].b;
         const double2 w = s_wv[lane], sig = s_sv[lane];
         const double yp0 = on0 ? fmax(0.0, yc.x + sig.x * (bi - ax0)) : 0.0;
         const double yp1 = on1 ? fmax(0.0, yc.y + sig.y * (bi - ax1)) : 0.0;
@@ -932,24 +903,24 @@ k_dual2(const DevProb P, const DevState S, const int it, const int rows_per_cta,
         }
     };
     if (coop) {                                                // warp 0, the chunk's one row
-        trip(0, [&](int, int, double& ax0, double& ax1) { ax0 = cg0; ax1 = cg1; });
+        trip(0, rc, [&](int, int, int, double& ax0, double& ax1) { ax0 = cg0; ax1 = cg1; });
         return;
     }
     // as in k_primal2: the shared / global choice of the entries is made once per CTA
-    const int ntrips = frz ? s_nrows : r1 - r0;                // a frozen row's multiplier rests at zero for the whole tile
+    const int ntrips = frz ? hd.y : r1 - r0;                   // a frozen row's multiplier rests at zero for the whole tile
     if (sl.se) {
         const int4* const E = sl.se - sl.base;
         for (int k = warp; k < ntrips; k += kWarps)
-            trip(k, [&](const int k_, const int lr, double& ax0, double& ax1) {
-                ax0 = ax1 = DualRowScalars::View(rows_per_cta, cap).rcs[k_];   // rconst of the row, 0 without frozen coordinates
-                dot2_entries<true, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.xbar, ax0, ax1, kBlk, xoff);
+            trip(k, row_at(k), [&](const int k_, const int p0, const int p1, double& ax0, double& ax1) {
+                ax0 = ax1 = reinterpret_cast<const DualRec*>(row_scalar_smem(rows_per_cta, cap))[k_].rc;   // 0 without frozen coordinates
+                dot2_entries<true, unsigned, false>(E, p0, p1, S.xbar, ax0, ax1, kBlk, xoff);
             });
     } else {
         const int4* const E = reinterpret_cast<const int4*>(aent);
         for (int k = warp; k < ntrips; k += kWarps)
-            trip(k, [&](const int k_, const int lr, double& ax0, double& ax1) {
-                ax0 = ax1 = DualRowScalars::View(rows_per_cta, cap).rcs[k_];
-                dot2_entries<false, unsigned, false>(E, sl.sp[lr], frz ? s_ends[lr] : sl.sp[lr + 1], S.xbar, ax0, ax1, kBlk, xoff);
+            trip(k, row_at(k), [&](const int k_, const int p0, const int p1, double& ax0, double& ax1) {
+                ax0 = ax1 = reinterpret_cast<const DualRec*>(row_scalar_smem(rows_per_cta, cap))[k_].rc;
+                dot2_entries<false, unsigned, false>(E, p0, p1, S.xbar, ax0, ax1, kBlk, xoff);
             });
     }
 }
@@ -1357,9 +1328,8 @@ k_freeze_rows(const DevProb P, const DevState S, const FreezeArgs F, const int r
 
 // Folded matrices of every tile with a running node, from the flags (see DevState). One thread per column / row.
 //   k_fold_cols: which columns rest at ONE value for the whole tile (both blocks flag 3 with equal values, a block
-//                without a running node agrees) — their contribution to A x is a per-row constant of the tile
-//   k_fold_A:    per row of A the entries of the other columns, packed; rconst = sum over the folded ones
-//   k_fold_AT:   per row of A' (column of A) the entries whose row is not frozen (a frozen row's multiplier is zero)
+//                without a running node agrees) — their contribution to A x is a per-row constant of the tile —
+//                and which columns (ftc) and rows (ftr) are frozen for the tile; the work lists (k_work_*) follow
 // running nodes of the tile's two 32-node blocks -> s_l[0], s_l[1] (all threads of the CTA call; ends with a barrier)
 __device__ __forceinline__ void tile_running(const DevState& S, const int tile, int* s_l) {
     if (threadIdx.x < kBlk) {
@@ -1392,49 +1362,176 @@ k_fold_cols(const DevProb P, const DevState S) {
         S.ftr[(size_t)tile * P.m + i] = (l0 == 0 || g0[i] != 0) && (l1 == 0 || g0[P.m + i] != 0);
 }
 
+// Work lists of the frozen-path step kernels (WorkList), built after k_fold_cols for every tile with a running node.
+// PRIMAL: rows of A' (columns j, active unless ftc, entry (j, i) kept unless row i is frozen: its multiplier is zero);
+// dual: rows of A (rows i, active unless ftr, entry (i, j) kept unless column j is folded into rconst).
+//   k_work_count: kept entries of every row, -1 for a frozen one. One thread per row.
+//   k_work_scan:  one CTA per tile: the active rows' places and entry starts, then the chunk headers.
+//   k_work_fill:  the kept entries (in the row's order) and the record of every active row. One thread per row.
+template <bool PRIMAL>
+__device__ __forceinline__ bool work_row_active(const DevState& S, const int rows, const int tile, const int r) {
+    return !(PRIMAL ? S.ftc : S.ftr)[(size_t)tile * rows + r];
+}
+template <bool PRIMAL>
+__device__ __forceinline__ bool work_entry_kept(const DevProb& P, const DevState& S, const int tile, const int col) {
+    return PRIMAL ? !S.ftr[(size_t)tile * P.m + col] : !S.fcol[(size_t)tile * P.n + col];
+}
+
+template <bool PRIMAL>
 __global__ void __launch_bounds__(kCtaThreads)
-k_fold_A(const DevProb P, const DevState S) {
+k_work_count(const DevProb P, const DevState S) {
     __shared__ int s_l[2];
     const int tile = blockIdx.y;
     tile_running(S, tile, s_l);
     if (s_l[0] + s_l[1] == 0) return;
-    const uint8_t* __restrict__ fcol = S.fcol + (size_t)tile * P.n;
-    const double* __restrict__ fval = S.fval + (size_t)tile * P.n;
-    int4* __restrict__ out = reinterpret_cast<int4*>(S.fentA + (size_t)tile * P.nnz);
-    const int4* __restrict__ in = reinterpret_cast<const int4*>(P.ent);
-    for (int i = blockIdx.x * kCtaThreads + threadIdx.x; i < P.m; i += gridDim.x * kCtaThreads) {
-        const int p0 = __ldg(P.rowptr + i), p1 = __ldg(P.rowptr + i + 1);
-        int w = p0;
-        double c = 0.0;
-        for (int p = p0; p < p1; ++p) {
-            const int4 e = __ldg(in + p);
-            if (fcol[e.x]) c = fma(__hiloint2double(e.w, e.z), fval[e.x], c);
-            else out[w++] = e;
+    const int rows = PRIMAL ? P.n : P.m;
+    const int32_t* __restrict__ ptr = PRIMAL ? P.cptr : P.rowptr;
+    const Ent* __restrict__ ent = PRIMAL ? P.cent : P.ent;
+    int32_t* __restrict__ kept = (PRIMAL ? S.wlC : S.wlR).kept + (size_t)tile * rows;
+    for (int r = blockIdx.x * kCtaThreads + threadIdx.x; r < rows; r += gridDim.x * kCtaThreads) {
+        int cnt = -1;
+        if (work_row_active<PRIMAL>(S, rows, tile, r)) {
+            cnt = 0;
+            for (int p = __ldg(ptr + r); p < __ldg(ptr + r + 1); ++p) cnt += work_entry_kept<PRIMAL>(P, S, tile, __ldg(&ent[p].idx));
         }
-        S.fendA[(size_t)tile * P.m + i] = w;
-        S.rconst[(size_t)tile * P.m + i] = c;
+        kept[r] = cnt;
     }
 }
 
+// Chunk headers: the long active rows (more than kLongRow stored entries, the rows the full-matrix plan gives a chunk
+// of their own) take chunks 0 .. L-1, one each; the N other active rows are split over the remaining Q chunks in row
+// order, chunk q holding the rows whose weight prefix P_s (kept entries + cw per row) lies in [q W / Q, (q+1) W / Q),
+// W the total. A row's trip costs about one round trip per BLP_U kept entries plus one for its state, hence
+// cw >= BLP_U; cw >= E / (Q rows_per_cta - N) (E: kept entries of the N rows) bounds every chunk to rows_per_cta rows.
+// Q >= N / rows_per_cta and Q >= 1 when N > 0: the full-matrix plan has at least that many chunks of short rows.
+template <bool PRIMAL>
+__global__ void __launch_bounds__(1024)
+k_work_scan(const DevProb P, const DevState S, const int chunks, const int rows_per_cta) {
+    __shared__ int s_l[2];
+    __shared__ int4 s_part[32];
+    const int tile = blockIdx.x;
+    tile_running(S, tile, s_l);
+    if (s_l[0] + s_l[1] == 0) return;
+    const WorkList& W = PRIMAL ? S.wlC : S.wlR;
+    const int rows = PRIMAL ? P.n : P.m;
+    const int32_t* __restrict__ ptr = PRIMAL ? P.cptr : P.rowptr;
+    int32_t* const kept = W.kept + (size_t)tile * rows;
+    int2* const out = W.row + (size_t)tile * (rows + 1);
+    int4* const hdr = W.chunk + (size_t)tile * rows;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int seg = (rows + blockDim.x - 1) / blockDim.x;
+    const int r0 = min(rows, (int)threadIdx.x * seg), r1 = min(rows, r0 + seg);
+    // (long rows, their kept entries, other rows, their kept entries) of the thread's segment
+    int4 c = make_int4(0, 0, 0, 0);
+#pragma unroll 4
+    for (int r = r0; r < r1; ++r) {
+        const int k = kept[r];
+        const bool lng = __ldg(ptr + r + 1) - __ldg(ptr + r) > kLongRow;
+        if (k >= 0 && lng) c.x += 1, c.y += k;
+        if (k >= 0 && !lng) c.z += 1, c.w += k;
+    }
+    // exclusive scan over the threads, in thread (= row) order
+    int4 inc = c;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int x = __shfl_up_sync(0xffffffffu, inc.x, d), y = __shfl_up_sync(0xffffffffu, inc.y, d);
+        const int z = __shfl_up_sync(0xffffffffu, inc.z, d), w = __shfl_up_sync(0xffffffffu, inc.w, d);
+        if (lane >= d) inc.x += x, inc.y += y, inc.z += z, inc.w += w;
+    }
+    if (lane == 31) s_part[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        int4 v = lane < (int)(blockDim.x >> 5) ? s_part[lane] : make_int4(0, 0, 0, 0);
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int x = __shfl_up_sync(0xffffffffu, v.x, d), y = __shfl_up_sync(0xffffffffu, v.y, d);
+            const int z = __shfl_up_sync(0xffffffffu, v.z, d), w = __shfl_up_sync(0xffffffffu, v.w, d);
+            if (lane >= d) v.x += x, v.y += y, v.z += z, v.w += w;
+        }
+        s_part[lane] = v;                                      // inclusive over warps 0 .. lane
+    }
+    __syncthreads();
+    const int4 tot = s_part[31];
+    int4 run = make_int4(inc.x - c.x, inc.y - c.y, inc.z - c.z, inc.w - c.w);
+    if (warp > 0) {
+        const int4 b = s_part[warp - 1];
+        run.x += b.x, run.y += b.y, run.z += b.z, run.w += b.w;
+    }
+    const int L = tot.x, EL = tot.y, N = tot.z;
+    for (int r = r0; r < r1; ++r) {
+        const int k = kept[r];
+        if (k < 0) continue;
+        if (__ldg(ptr + r + 1) - __ldg(ptr + r) > kLongRow) {
+            out[run.x] = make_int2(r, run.y);
+            run.x += 1, run.y += k;
+        } else {
+            out[L + run.z] = make_int2(r, EL + run.w);
+            run.z += 1, run.w += k;
+        }
+    }
+    if (threadIdx.x == 0) {
+        out[L + N] = make_int2(-1, EL + tot.w);
+        W.count[tile] = L + N;
+    }
+    __syncthreads();                                           // out[] complete, kept[] free: it holds chunk starts now
+    for (int q = threadIdx.x; q < L; q += blockDim.x) hdr[q] = make_int4(q, -1, out[q].y, out[q + 1].y);
+    const int Q = chunks - L;
+    if (Q < 1) return;
+    const long long ES = tot.w, room = (long long)Q * rows_per_cta - N;
+    const bool by_count = room <= 0 || ES / room >= (1 << 16);   // then every row weighs the same (Q rows_per_cta >= N)
+    const long long cw = by_count ? 1 : max((long long)BLP_U, (ES + room - 1) / room);
+    const unsigned long long Wt = (by_count ? 0 : ES) + cw * N;
+    auto chunk_of = [&](const int s) -> int {                  // s < N
+        const unsigned long long pw = (by_count ? 0 : out[L + s].y - EL) + cw * s;
+        return (int)((unsigned __int128)pw * Q / Wt);
+    };
+    // chunk q starts at the first row s with chunk_of(s) >= q
+    for (int s = threadIdx.x; s <= N; s += blockDim.x) {
+        const int qs = s < N ? chunk_of(s) : Q, qp = s > 0 ? chunk_of(s - 1) : -1;
+        for (int q = qp + 1; q <= qs && q < Q; ++q) kept[q] = s;
+    }
+    __syncthreads();
+    for (int q = threadIdx.x; q < Q; q += blockDim.x) {
+        const int k0 = L + kept[q], k1 = L + (q + 1 < Q ? kept[q + 1] : N);
+        hdr[L + q] = make_int4(k0, k1 - k0, out[k0].y, out[k1].y);
+    }
+}
+
+template <bool PRIMAL>
 __global__ void __launch_bounds__(kCtaThreads)
-k_fold_AT(const DevProb P, const DevState S) {
+k_work_fill(const DevProb P, const DevState S) {
     __shared__ int s_l[2];
     const int tile = blockIdx.y;
     tile_running(S, tile, s_l);
-    const int l0 = s_l[0], l1 = s_l[1];
-    if (l0 + l1 == 0) return;
-    const uint8_t* __restrict__ f0 = S.rfrz + (size_t)(2 * tile) * P.m;
-    int4* __restrict__ out = reinterpret_cast<int4*>(S.fentAT + (size_t)tile * P.nnz);
-    const int4* __restrict__ in = reinterpret_cast<const int4*>(P.cent);
-    for (int j = blockIdx.x * kCtaThreads + threadIdx.x; j < P.n; j += gridDim.x * kCtaThreads) {
-        const int p0 = __ldg(P.cptr + j), p1 = __ldg(P.cptr + j + 1);
-        int w = p0;
-        for (int p = p0; p < p1; ++p) {
-            const int4 e = __ldg(in + p);
-            const bool frozen = (l0 == 0 || f0[e.x] != 0) && (l1 == 0 || f0[P.m + e.x] != 0);
-            if (!frozen) out[w++] = e;
+    if (s_l[0] + s_l[1] == 0) return;
+    const WorkList& W = PRIMAL ? S.wlC : S.wlR;
+    const int rows = PRIMAL ? P.n : P.m;
+    const int32_t* __restrict__ ptr = PRIMAL ? P.cptr : P.rowptr;
+    const int4* __restrict__ in = reinterpret_cast<const int4*>(PRIMAL ? P.cent : P.ent);
+    const int2* __restrict__ act = W.row + (size_t)tile * (rows + 1);
+    int4* __restrict__ out = reinterpret_cast<int4*>(W.ent + (size_t)tile * P.nnz);
+    const int nact = W.count[tile];
+    for (int k = blockIdx.x * kCtaThreads + threadIdx.x; k < nact; k += gridDim.x * kCtaThreads) {
+        const int2 v = act[k];
+        const int r = v.x, p0 = __ldg(ptr + r), p1 = __ldg(ptr + r + 1);
+        int w = v.y;
+        if constexpr (PRIMAL) {
+            for (int p = p0; p < p1; ++p) {
+                const int4 e = __ldg(in + p);
+                if (work_entry_kept<true>(P, S, tile, e.x)) out[w++] = e;
+            }
+            PrimalRowScalars(P, S, 2 * tile, reinterpret_cast<PrimalRec*>(W.rec) + (size_t)tile * rows)(r, k);
+        } else {
+            const uint8_t* __restrict__ fcol = S.fcol + (size_t)tile * P.n;
+            const double* __restrict__ fval = S.fval + (size_t)tile * P.n;
+            double c = 0.0;                                    // rconst: sum over the folded columns, in row order
+            for (int p = p0; p < p1; ++p) {
+                const int4 e = __ldg(in + p);
+                if (fcol[e.x]) c = fma(__hiloint2double(e.w, e.z), fval[e.x], c);
+                else out[w++] = e;
+            }
+            reinterpret_cast<DualRec*>(W.rec)[(size_t)tile * rows + k] = DualRec{__ldg(P.b + r), c};
         }
-        S.fendAT[(size_t)tile * P.n + j] = w;
     }
 }
 
